@@ -131,7 +131,10 @@ __global__ void __launch_bounds__(D2D_BLOCK_THREADS) d2d_step_block_generic_kern
             if (active) {
                 const uint32_t rbkey = key & 0x1fffffffu;
                 const int b = rbkey % (uint32_t)nbins, beg = S.bin_off[b], end = beg + S.bin_cnt[b];
-                float I = 0.0f, dmin2 = 3.0e38f;
+                // the sum is accumulated in fp64: an RB may hold over a thousand links, and an fp32 running sum of n terms drifts by
+                // ~sqrt(n) ulp - at n = 1 100, 1e-4 relative of a SINR just outside the 0.0625 dB band of the fp64 pass (DESIGN.md 4.4)
+                double Id = 0.0;
+                float dmin2 = 3.0e38f;
                 bool side = false;
                 for (int q = beg; q < end; ++q) {
                     const int k = S.sorted[q];
@@ -139,7 +142,7 @@ __global__ void __launch_bounds__(D2D_BLOCK_THREADS) d2d_step_block_generic_kern
                     if (k != j && (__float_as_uint(rk.w) & 0x9fffffffu) == rbkey) {
                         const float dx = rk.x - xj.x, dy = rk.y - xj.y;
                         const float d2 = fmaf(dx, dx, dy * dy);
-                        I = fmaf(rk.z, d2d_gain<PLE2>(d2, P.neg_half_ple) * d2d_shadow_factor(P, d2, genv, (uint32_t)j, (uint32_t)k, 0), I);
+                        Id += (double)(rk.z * (d2d_gain<PLE2>(d2, P.neg_half_ple) * d2d_shadow_factor(P, d2, genv, (uint32_t)j, (uint32_t)k, 0)));
                         dmin2 = fminf(dmin2, d2);
                         side |= (__float_as_uint(rk.w) >> 29) & 1u;
                     }
@@ -149,7 +152,7 @@ __global__ void __launch_bounds__(D2D_BLOCK_THREADS) d2d_step_block_generic_kern
                 const float dx = rj.x - xj.x, dy = rj.y - xj.y;
                 const float d2own = fmaf(dx, dx, dy * dy);
                 const float gown = d2d_gain<PLE2>(d2own, P.neg_half_ple);
-                o = d2d_link_epilogue<PLE2>(p, xj.z, gown, gown * d2d_shadow_factor(P, d2own, genv, (uint32_t)j, (uint32_t)j, 0), I, Av, sb, P);
+                o = d2d_link_epilogue<PLE2>(p, xj.z, gown, gown * d2d_shadow_factor(P, d2own, genv, (uint32_t)j, (uint32_t)j, 0), (float)Id, Av, sb, P);
                 if (P.shadow_chi_dB > 0.f && d2own > P.shadow_d0sq)      // the SNR's own evaluation of the path loss (simulator.py:113)
                     o.snr_dB -= P.shadow_chi_dB * d2d_shadow_normal(P, genv, (uint32_t)j, (uint32_t)j, 1);
                 if (D2D_RESCUE_ENABLED && d2d_needs_rescue<true>(o, fminf(dmin2, d2own), P)) {   // rare: fp64 pass (d2d_common.cuh)
@@ -364,23 +367,25 @@ __global__ void __launch_bounds__(D2D_BLOCK_THREADS, LPT <= 2 ? 4 : 3) d2d_step_
             const uint32_t j = tid + k * D2D_BLOCK_THREADS;
             D2DLinkOut o = {0.f, 0.f, 0.f, 0.f};
             if (live[k]) {
-                float I = 0.0f, dmin2 = 3.0e38f;
+                // fp64 accumulation, as in the general kernel: an RB may hold all 1024 links of an env
+                double Id = 0.0;
+                float dmin2 = 3.0e38f;
                 if (cue[k] && !P.pos64) {
                     for (uint32_t q = beg[k]; q < end[k]; ++q)
-                        if (q != self[k]) I += rec[q].w;
+                        if (q != self[k]) Id += (double)rec[q].w;
                 } else {
                     for (uint32_t q = beg[k]; q < end[k]; ++q) {
                         if (q == self[k]) continue;
                         const float4 rk = rec[q];
                         const float dx = rk.x - rx[k].x, dy = rk.y - rx[k].y;
                         const float d2 = fmaf(dx, dx, dy * dy);
-                        I = fmaf(rk.z, d2d_gain<PLE2>(d2, P.neg_half_ple), I);
+                        Id += (double)(rk.z * d2d_gain<PLE2>(d2, P.neg_half_ple));
                         dmin2 = fminf(dmin2, d2);
                     }
                 }
                 const float dxo = tx[k].x - rx[k].x, dyo = tx[k].y - rx[k].y;
                 const float2 sBk = link_sB(j, cue[k]);
-                o = d2d_link_epilogue<PLE2>((int)pw[k], pl[k], gown[k], gown[k], I, link_cA(j, cue[k]), sBk, P);
+                o = d2d_link_epilogue<PLE2>((int)pw[k], pl[k], gown[k], gown[k], (float)Id, link_cA(j, cue[k]), sBk, P);
                 uint32_t qslot = D2D_BLOCK_RESQ;
                 const bool need = D2D_RESCUE_ENABLED && d2d_needs_rescue<true>(o, fminf(dmin2, fmaf(dxo, dxo, dyo * dyo)), P);
                 if (need) {

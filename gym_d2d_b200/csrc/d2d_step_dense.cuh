@@ -29,6 +29,7 @@
 
 #define D2D_DENSE_MAX_LPT 5
 #define D2D_DENSE_MAX_WARPS 16
+#define D2D_DENSE_WALK_BAND_DB 0.0075f      // rescue band per sqrt(peer) of a long walk: 2 sqrt(n) ulp of SINR, 1.45x margin to 1e-4
 // blocks per SM the register allocation has to allow (80 registers at 256 threads)
 #define D2D_DENSE_MINB(BT) ((BT) <= 128 ? 6 : (BT) <= 160 ? 5 : (BT) <= 192 ? 4 : 3)
 
@@ -446,6 +447,9 @@ __global__ void __launch_bounds__(BT, D2D_DENSE_MINB(BT)) d2d_step_dense_kernel(
                 sBk = link_sB(j, cue[k]);
                 o = d2d_link_epilogue<PLE2>((int)pwk, pwr[pwk] /* 10^(p/10) again: a table read costs less than a register held across the barrier */, gown, gown, I, link_cA(j, cue[k]), sBk, P);
                 need = D2D_RESCUE_ENABLED && d2d_needs_rescue<EXACT, !FULL>(o, fminf(dmin2, d2own[k]), P);
+                // the fp32 running sum over n peers drifts by ~sqrt(n) ulp: on crowded RBs the band widens with the walk
+                // (n = 1024: 0.24 dB, where the pass still rewrites the SINR; DESIGN.md 4.4)
+                if (D2D_RESCUE_ENABLED && n > 64u && fabsf(o.sinr_dB) < D2D_DENSE_WALK_BAND_DB * sqrtf((float)n)) need = true;
             }
             if (lv) {
                 cap_part += o.cap;

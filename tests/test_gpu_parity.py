@@ -48,18 +48,21 @@ CONFIGS = {
     'small': dict(num_rbs=3, num_cues=4, num_due_pairs=5),
     'cue_only': dict(num_rbs=4, num_cues=9, num_due_pairs=0),
     'due_only': dict(num_rbs=5, num_cues=0, num_due_pairs=12),
-    'warp_max': dict(num_rbs=16, num_cues=24, num_due_pairs=40),      # N = 64: both lane slots full
+    'warp_max': dict(num_rbs=64, num_cues=32, num_due_pairs=32),      # the warp kernel's limits: both lane slots full, 64 RBs
+    'dense_64_links': dict(num_rbs=16, num_cues=24, num_due_pairs=40),   # N = 64, but D > 32: the dense kernel (1 x 256)
     'block_min': dict(num_rbs=16, num_cues=25, num_due_pairs=40),     # N = 65: first block-kernel size
     'dense_small': dict(num_rbs=8, num_cues=6, num_due_pairs=30),
     'dense': dict(num_rbs=100, num_cues=100, num_due_pairs=500),
     'one_rb_crowded': dict(num_rbs=1, num_cues=20, num_due_pairs=30),  # every link interferes with every other
     'many_rbs_few_links': dict(num_rbs=100, num_cues=10, num_due_pairs=20),   # R > 64 with N <= 64
+    'sorting': dict(num_rbs=600, num_cues=80, num_due_pairs=320),     # R > 512: the sorting block kernel, 2 links per thread
+    'general': dict(num_rbs=25, num_cues=225, num_due_pairs=800),     # N = 1025: the general-topology kernel
     'one_power_level': dict(num_rbs=6, num_cues=8, num_due_pairs=8, cue_max_tx_power_dBm=0, due_max_tx_power_dBm=0),
 }
 
 
 @pytest.mark.parametrize('name,E', [('default', 512), ('tiny', 64), ('small', 128), ('cue_only', 64), ('due_only', 64),
-                                    ('warp_max', 96), ('block_min', 48), ('dense_small', 64), ('dense', 12),
+                                    ('warp_max', 96), ('dense_64_links', 96), ('block_min', 48), ('dense_small', 64), ('dense', 12),
                                     ('one_rb_crowded', 64), ('many_rbs_few_links', 64), ('one_power_level', 64)])
 def test_step_matches_oracle(name, E):
     kw = CONFIGS[name]

@@ -367,7 +367,7 @@ def test_per_agent_rewards_with_many_rbs(kind):
 
 
 # ---- per-agent reward thresholds decided in fp64 (VERDICT r1: the threshold neighbourhood used to be exempt) -------------------------
-@pytest.mark.parametrize('name', ['default', 'block_min', 'dense_small', 'one_rb_crowded'])
+@pytest.mark.parametrize('name', ['default', 'block_min', 'dense_small', 'one_rb_crowded', 'sorting', 'general'])
 @pytest.mark.parametrize('kind', ['shannon', 'cue_sinr_shannon'])
 def test_reward_threshold_a_hair_from_a_link_sinr(name, kind):
     """The threshold is placed 1e-9 dB above / below the float64 SINR of actual links - far inside fp32's resolution of a dB

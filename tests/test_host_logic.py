@@ -293,3 +293,79 @@ def test_dict_views_follow_the_reference_layout():
             assert all(isinstance(v, int) for v in acts[k])
         assert list(state['sinrs_db']) == [tuple(k.split(':')) for k in keys]
     assert len(env._views) == 2
+
+
+# ---- the step-kernel dispatch restated in tests/_kernel_dispatch.py, against the real host functions ---------------------------
+_LAYOUT_PROBE = r'''
+#include "d2d_internal.h"
+#include "d2d_step_dense.cuh"
+#include "d2d_step_block.cuh"
+#include "d2d_step_warp.cuh"
+#include <cstdio>
+int main() {
+    std::printf("rc %zu\n", sizeof(D2DDenseRC));
+    int N, R, V, bt;
+    while (std::scanf("%d %d %d %d", &N, &R, &V, &bt) == 4) {
+        const int cap = d2d_dense_bin_cap(N, R);
+        std::printf("%d %d %d %d %d %u %zu %zu %u %u %u\n", N, R, V, bt, cap, d2d_dense_layout(N, R, cap, bt, V).total,
+                    d2d_block2_smem_bytes(N, R), d2d_block_smem_bytes(N, R), d2d_warp_smem_bytes(R, 2), d2d_warp_smem_bytes(R, 4),
+                    d2d_warp_smem_bytes(R, 8));
+    }
+    return 0;
+}
+'''
+
+
+def test_restated_kernel_layouts_match_the_host_functions(tmp_path):
+    """tests/_kernel_dispatch.py restates the bin capacity and the shared-memory layouts of the dense, sorting, general and warp
+    kernels; the GPU matrix (tests/test_kernel_matrix.py) asserts step_geometry() against them.  Here the real host functions
+    (d2d_dense_bin_cap, d2d_dense_layout, d2d_block2_smem_bytes, d2d_block_smem_bytes, d2d_warp_smem_bytes) are compiled into a
+    host-only program and must agree byte for byte over a sweep of link and RB counts."""
+    import shutil
+    import subprocess
+    from tests import _kernel_dispatch as KD
+    nvcc = shutil.which('nvcc') or ('/usr/local/cuda/bin/nvcc' if Path('/usr/local/cuda/bin/nvcc').exists() else None)
+    if nvcc is None:
+        pytest.skip('nvcc not found')
+    src = tmp_path / 'layout_probe.cu'
+    src.write_text(_LAYOUT_PROBE)
+    exe = tmp_path / 'layout_probe'
+    subprocess.run([nvcc, '-gencode', 'arch=compute_100a,code=sm_100a', '-std=c++17', '-diag-suppress', '159',
+                    '-I', str(ROOT / 'gym_d2d_b200' / 'csrc'), '-o', str(exe), str(src)], check=True, capture_output=True)
+    cases = []
+    for N in (1, 64, 65, 100, 255, 256, 257, 300, 320, 321, 512, 600, 640, 641, 700, 768, 769, 800, 960, 961, 1000, 1024, 1025,
+              2000, 3000, 3300, 4000):
+        for R in (1, 4, 25, 64, 100, 300, 512, 600, 3000):
+            for D in {0, N // 5, (4 * N) // 5, N}:
+                cases.append((N, R, 1 + N + D, 256 if (N + R + D) % 2 else 320))
+    res = subprocess.run([str(exe)], input=''.join(f'{n} {r} {v} {b}\n' for n, r, v, b in cases), check=True, capture_output=True, text=True)
+    lines = res.stdout.strip().splitlines()
+    assert lines[0] == f'rc {KD.DENSE_RC_BYTES}'
+    assert len(lines) == 1 + len(cases)
+    for (N, R, V, bt), line in zip(cases, lines[1:]):
+        got = [int(x) for x in line.split()]
+        assert got[:4] == [N, R, V, bt]
+        cap = KD.dense_bin_cap(N, R)
+        want = [cap, KD.dense_smem(N, R, cap, bt, V), KD.block2_smem(N, R), KD.block_smem(N, R),
+                KD.warp_smem(R, 2), KD.warp_smem(R, 4), KD.warp_smem(R, 8)]
+        assert got[4:] == want, (N, R, V, bt)
+
+
+@pytest.mark.parametrize('R,C,D,E,env,family,lpt,bt,wpb', [
+    (64, 32, 32, 1024, {}, 'warp', 0, 0, 2), (64, 32, 32, 5000, {}, 'warp', 0, 0, 4),
+    (64, 32, 32, 100, {'D2D_B200_WPB': '8'}, 'warp', 0, 0, 8), (16, 24, 40, 96, {}, 'dense', 1, 256, 0),
+    (65, 32, 32, 64, {}, 'dense', 1, 256, 0), (64, 33, 32, 64, {}, 'dense', 1, 256, 0),
+    (50, 60, 240, 64, {}, 'dense', 1, 320, 0), (40, 80, 320, 64, {}, 'dense', 2, 256, 0), (60, 100, 500, 64, {}, 'dense', 2, 320, 0),
+    (30, 140, 560, 64, {}, 'dense', 3, 256, 0), (25, 160, 640, 64, {}, 'dense', 3, 320, 0), (25, 224, 800, 64, {}, 'dense', 4, 256, 0),
+    (600, 40, 160, 64, {}, 'sorting', 1, 0, 0), (300, 100, 500, 64, {}, 'sorting', 3, 0, 0), (600, 224, 800, 64, {}, 'sorting', 4, 0, 0),
+    (60, 100, 500, 64, {'D2D_B200_DENSE': '0'}, 'sorting', 3, 0, 0), (25, 225, 800, 64, {}, 'general', 0, 0, 0),
+    (100, 600, 2400, 64, {}, 'general', 0, 0, 0), (100, 800, 3200, 64, {}, 'unsupported', 0, 0, 0)])
+def test_restated_dispatch_picks_the_documented_family(R, C, D, E, env, family, lpt, bt, wpb):
+    """Spot checks of the restated dispatch at the edges of each family: C, D <= 32 and R <= 64 for the warp kernel; N = 1024
+    as the largest dense / sorting shape; R > 512 or a dense layout over 75 KB for the sorting kernel; past 227 KB refused."""
+    from tests._kernel_dispatch import expected_kernel
+    k = expected_kernel(dict(num_rbs=R, num_cues=C, num_due_pairs=D), E, env=env)
+    assert (k['family'], k['lpt'], k['bt'], k['wpb']) == (family, lpt, bt, wpb)
+    assert expected_kernel(dict(num_rbs=4, num_cues=5, num_due_pairs=6), 64, env={}, downlink=True)['family'] == 'general'
+    assert expected_kernel(dict(num_rbs=25), 512, env={})['spec'] and not expected_kernel(dict(num_rbs=25), 512, env={'D2D_B200_SPEC': '0'})['spec']
+    assert expected_kernel(dict(num_rbs=100, num_cues=100, num_due_pairs=500), 64, env={})['spec']
