@@ -128,10 +128,12 @@ struct D2DParams {
 
 #ifdef D2D_TIMELINE
 // Instrumented build only: every warp of the warp kernel stamps (globaltimer at entry, clock64 at entry / before
-// griddepcontrol.wait / after it / at its end, SM id) so that profiles/timeline.py can lay consecutive launches side by side.
+// griddepcontrol.wait / after it / at its end, SM id) so that profiles/timeline.py can lay consecutive launches side by side,
+// and counts what the warp did: envs stepped, flagged links recomputed in fp64 before / after its wait, envs that took the
+// all-pairs overflow path.
 #define D2D_TL_SLOTS 64
 #define D2D_TL_WARPS 4096
-struct D2DTlRec { unsigned long long g0, c0, c1, c2, c3, smid; };
+struct D2DTlRec { unsigned long long g0, c0, c1, c2, c3, smid, n_env, n_pre, n_post, n_ovf; };
 __device__ D2DTlRec d2d_tl_buf[D2D_TL_SLOTS][D2D_TL_WARPS];
 __device__ __forceinline__ unsigned long long d2d_tl_clock() { return (unsigned long long)clock64(); }
 __device__ __forceinline__ unsigned long long d2d_tl_gtime() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }

@@ -328,6 +328,9 @@ __device__ __forceinline__ D2DLinkOut d2d_link_epilogue_warp(bool live, float p_
 
 // Some RB holds more links than a bin has record slots: all-pairs pass over the 64 link slots by shuffle (no table).
 // A term counts when the RB keys match and it is not the victim itself.  Returns (I_A, I_B, dmin2_A, dmin2_B).
+// Only lanes with a live link are visited, in lane order: a lane whose two slots are both dead (inactive keys, unique per lane
+// and slot) matches no victim but itself, so every term it would add is exactly 0.0f and skipping it changes no bit.  In a late
+// launch this path is on the last warp to reach the wait in almost every launch of a one-wave batch (profiles/timeline.py).
 #ifndef D2D_RARE_ATTR
 #define D2D_RARE_ATTR __forceinline__     // A/B knob: __noinline__ moves the rare paths out of the hot loop's code
 #endif
@@ -336,7 +339,8 @@ __device__ D2D_RARE_ATTR float4 d2d_all_pairs_warp(uint32_t lane, uint32_t keyA,
                                                       float nhp) {
     float IA = 0.f, IB = 0.f, dminA = 3.0e38f, dminB = 3.0e38f;
 #pragma unroll 1
-    for (uint32_t k = 0; k < 32u; ++k) {
+    for (uint32_t src = __ballot_sync(0xffffffffu, (keyA & keyB & D2D_INACTIVE_KEY) == 0u); src; src &= src - 1u) {
+        const uint32_t k = (uint32_t)__ffs((int)src) - 1u;
         const uint32_t kA = __shfl_sync(0xffffffffu, keyA, k), kB = __shfl_sync(0xffffffffu, keyB, k);
         const float4 ra = make_float4(__shfl_sync(0xffffffffu, recA.x, k), __shfl_sync(0xffffffffu, recA.y, k),
                                       __shfl_sync(0xffffffffu, recA.z, k), __shfl_sync(0xffffffffu, recA.w, k));
@@ -499,6 +503,8 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
 #ifdef D2D_TIMELINE
     const unsigned long long tl_g0 = d2d_tl_gtime(), tl_c0 = d2d_tl_clock();
     unsigned long long tl_c1 = 0, tl_c2 = 0;
+    uint32_t tl_env = 0, tl_pre = 0, tl_post = 0, tl_ovf = 0;      // envs, fp64 links before / after the wait, overflow envs
+    bool tl_waited = false;
 #endif
     d2d_pdl_entry(P.flags);
     uint32_t blk = (uint32_t)__cvta_generic_to_shared(d2d_warp_smem);
@@ -660,6 +666,9 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
             const uint32_t keyA = liveA ? rbA : (D2D_INACTIVE_KEY | lane), keyB = liveB ? rbB : (D2D_INACTIVE_KEY | 32u | lane);
             const float4 r = d2d_all_pairs_warp<PLE2, EXACT>(lane, keyA, keyB, make_float4(tA.x, tA.y, wA, uA), pB, wB, uB, P.neg_half_ple);
             IA = r.x; IB = r.y; dminA = r.z; dminB = r.w;
+#ifdef D2D_TIMELINE
+            ++tl_ovf;
+#endif
         } else {
             // bit t of valid <=> record t of the victim's bin exists and is not the victim (dead lane: 0)
             const uint32_t validA = liveA ? (((1u << nA) - 1u) ^ (1u << rankA)) : 0u;
@@ -694,6 +703,9 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
             const uint32_t keyA = liveA ? rbA : (D2D_INACTIVE_KEY | lane), keyB = liveB ? rbB : (D2D_INACTIVE_KEY | 32u | lane);
             const uint32_t nr = (uint32_t)d2d_rescue_warp<PLE2, EXACT, SPEC, false, !FULL>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_, tA, pB, oA, oB);
             st_resc += (ep_reset && t == 0u) ? 0u : nr;            // the reset step enters no statistic
+#ifdef D2D_TIMELINE
+            (tl_waited ? tl_post : tl_pre) += nr;
+#endif
         }
 
         // ---- per-warp statistics; flushed with the warp's LAST env, ahead of the wait and of that env's stores: the reductions
@@ -738,6 +750,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
         }
 #ifdef D2D_TIMELINE
         if (e == e0 && t == 0u) tl_c2 = d2d_tl_clock();
+        if (e == e0 && t == 0u && !LATE) tl_waited = true;
 #endif
 #ifdef D2D_EXPERIMENT_NOCOUNT     // A/B only: how much of the post-wait tail is the step-counter load
         ns_keep = 0;
@@ -789,6 +802,26 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
                 if (P.pwr_out) P.pwr_out[jB] = (int16_t)(liveB ? pB_ : 0u);
             }
         }
+
+        // ---- the other shapes: the rare fp64 pass after the env's per-link stores (it overwrites them) ---------------------------
+        const auto rescue_late = [&]() {
+            if (D2D_RESCUE_ENABLED && !RESCUE_EARLY && __any_sync(0xffffffffu, needA || needB)) {
+                const uint32_t keyA = liveA ? rbA : (D2D_INACTIVE_KEY | lane), keyB = liveB ? rbB : (D2D_INACTIVE_KEY | 32u | lane);
+                const uint32_t nr = (uint32_t)d2d_rescue_warp_late<PLE2, EXACT, SPEC, !FULL>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_, tA, pB);
+                st_resc += (ep_reset && t == 0u) ? 0u : nr;
+#ifdef D2D_TIMELINE
+                (tl_waited ? tl_post : tl_pre) += nr;
+#endif
+            }
+        };
+        // d2d_step: right here, before the group end.  A late launch stored the per-link outputs ahead of the wait, so the pass of
+        // the env that closes the warp's first group runs ahead of it too: after the wait it was on the critical path of every
+        // back-to-back launch of a one-wave batch (profiles/timeline.py).  Its count goes out with the warp's last env, not at the
+        // exit, where an outstanding atomic holds the warp's block slot.  (The multi-step modes keep the pass after the group's
+        // scalars and the count at the exit: measured faster for d2d_rollout, which has no wait in its loop.)
+        if (!MANY) rescue_late();
+        if (!MANY && FLUSH_EARLY && !RESCUE_EARLY && P.stats && e + 1u == e_end && lane == 5u && st_resc != 0u)
+            atomicAdd(P.stats + ((blockIdx.x * WPB + warp) % D2D_STATS_REPLICAS) * 8 + 5u, (double)st_resc);
         if (MANY && T <= 32u) {
             // per-step scalars: lane t keeps slice t's reward until the env's last step, then T lanes store their slices at once
             // (two strided stores per env instead of two single-lane stores per step)
@@ -822,7 +855,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
 #endif
                 if (e - g == e0) d2d_pdl_wait();                       // (the warp's first group: once per warp)
 #ifdef D2D_TIMELINE
-                if (e - g == e0) tl_c2 = d2d_tl_clock();
+                if (e - g == e0) { tl_c2 = d2d_tl_clock(); tl_waited = true; }
 #endif
 #ifdef D2D_EXPERIMENT_NOCOUNT
                 ns_keep = 0;
@@ -840,12 +873,10 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
             }
         }
 
-        // ---- throughput shape: the rare fp64 pass after the env's outputs are stored (it overwrites them) -------------------
-        if (D2D_RESCUE_ENABLED && !RESCUE_EARLY && __any_sync(0xffffffffu, needA || needB)) {
-            const uint32_t keyA = liveA ? rbA : (D2D_INACTIVE_KEY | lane), keyB = liveB ? rbB : (D2D_INACTIVE_KEY | 32u | lane);
-            const uint32_t nr = (uint32_t)d2d_rescue_warp_late<PLE2, EXACT, SPEC, !FULL>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_, tA, pB);
-            st_resc += (ep_reset && t == 0u) ? 0u : nr;
-        }
+        if (MANY) rescue_late();
+#ifdef D2D_TIMELINE
+        tl_env += last_t ? 1u : 0u;
+#endif
         if (last_t) {
             g = (g + 1u) & 31u;
             if (e + 1u == e_end) g = 0u;
@@ -870,6 +901,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
 #ifdef D2D_TIMELINE
     if (lane == 0u && blockIdx.x * WPB + warp < D2D_TL_WARPS) {
         D2DTlRec r; r.g0 = tl_g0; r.c0 = tl_c0; r.c1 = tl_c1; r.c2 = tl_c2; r.c3 = d2d_tl_clock(); r.smid = d2d_tl_smid();
+        r.n_env = tl_env; r.n_pre = tl_pre; r.n_post = tl_post; r.n_ovf = tl_ovf;
         d2d_tl_buf[P.tl_slot & (D2D_TL_SLOTS - 1)][blockIdx.x * WPB + warp] = r;
     }
 #endif
@@ -880,8 +912,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
             const double v = lane < 3u ? (double)vf : (double)vi;
             if (v != 0.0) atomicAdd(P.stats + ((blockIdx.x * WPB + warp) % D2D_STATS_REPLICAS) * 8 + lane, v);
         }
-    } else if (!RESCUE_EARLY && P.stats && lane == 5u && st_resc != 0u) {
-        // the one-wave shape runs the fp64 pass after the env's stores: its counter follows here (rarely non-zero for a one-env warp)
+    } else if (MANY && !RESCUE_EARLY && P.stats && lane == 5u && st_resc != 0u) {
         atomicAdd(P.stats + ((blockIdx.x * WPB + warp) % D2D_STATS_REPLICAS) * 8 + 5u, (double)st_resc);
     }
 }

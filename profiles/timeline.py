@@ -4,7 +4,10 @@ Needs the instrumented build (`nvcc ... -DD2D_TIMELINE`, see profiles/README.md)
 globaltimer + clock64 at entry, clock64 before / after griddepcontrol.wait and at its end, and its SM id.  The script replays
 a CUDA graph of 32 step launches (the bench's launch mode), reads the stamps of the last replay and prints, per launch, when
 its warps started / reached the wait / were released / ended - relative to the previous launch - i.e. how much of a step
-overlaps its predecessor under programmatic dependent launch.  Numbers from an instrumented build are not bench values.
+overlaps its predecessor under programmatic dependent launch.  Every warp also counts the envs it stepped, the flagged links it
+recomputed in fp64 before / after its wait and the envs that took the all-pairs overflow path; the script prints them for the
+last warp to reach the wait and the last to end, and splits the post-wait time by whether a warp ran an fp64 pass after its wait.
+Numbers from an instrumented build are not bench values.
 """
 import ctypes
 import sys
@@ -43,7 +46,7 @@ t.record()
 torch.cuda.synchronize()
 print(f'E={E}: {s.elapsed_time(t) * 1e3 / (20 * RING):.2f} us/step (instrumented build)  geom={env.step_geometry()}')
 
-buf = np.zeros((SLOTS, WARPS, 6), dtype=np.uint64)
+buf = np.zeros((SLOTS, WARPS, 10), dtype=np.uint64)
 geom = env.step_geometry()
 rc = lib.d2d_debug_timeline(buf.ctypes.data_as(ctypes.c_void_p), buf.nbytes, geom['block'] // 32)      # (one stamp table per warps-per-block shape)
 assert rc == 0
@@ -53,8 +56,8 @@ order = [(first_slot + k) % SLOTS for k in range(RING)]
 # last launch that stamped during the last replay (within 1 ms of the replay's first stamp)
 t_cut = int(buf[order[0], 0, 0]) - 1_000_000
 nw = int((buf[order[-1], :nw, 0].astype(np.int64) >= t_cut).sum()) or nw
-rec = buf[order, :nw].astype(np.int64)              # [launch][warp][g0, c0, c1, c2, c3, smid]
-g0, c0, c1, c2, c3, smid = (rec[..., i] for i in range(6))
+rec = buf[order, :nw].astype(np.int64)              # [launch][warp][g0, c0, c1, c2, c3, smid, n_env, n_pre, n_post, n_ovf]
+g0, c0, c1, c2, c3, smid, n_env, n_pre, n_post, n_ovf = (rec[..., i] for i in range(10))
 # clock64 is per SM: bring every SM onto the globaltimer axis with one offset per SM (SM clock = 1.965 GHz under load)
 GHZ = 1.965
 off = np.zeros(256)
@@ -86,4 +89,24 @@ print(f'  this first start - prev first start      {np.mean(t0[5:].min(1) - t0[4
 print(f'  this first start - prev last end         {np.mean(t0[5:].min(1) - t3[4:-1].max(1)) / 1e3:6.2f}  (negative = overlap)')
 print(f'  warps already at the wait when prev ends {np.mean([(t1[j] < t3[j - 1].max()).mean() for j in range(5, RING)]):6.2%}')
 print(f'  per-warp: start->wait {np.median(t1[k] - t0[k]) / 1e3:5.2f}  waiting {np.median(t2[k] - t1[k]) / 1e3:5.2f}  release->end {np.median(t3[k] - t2[k]) / 1e3:5.2f}')
+print(f'  last release -> last end                 {np.mean(t3[k].max(1) - t2[k].max(1)) / 1e3:6.2f}')
+
+# what the stragglers did: (envs, fp64 links before the wait, fp64 links after it, overflow envs) of the last warp at the wait and
+# of the last warp to end; post-wait time (release -> end) of the warps with and without an fp64 pass after their wait
+print('launch | last at wait: env pre post ovf | last to end: env pre post ovf | release->end [us] median / max: post-wait pass (n) | none (n)')
+attr = lambda k, w: f'{n_env[k, w]:3d} {n_pre[k, w]:3d} {n_post[k, w]:4d} {n_ovf[k, w]:3d}'
+for k in range(1, RING):
+    wa, we = int(t1[k].argmax()), int(t3[k].argmax())
+    post, m = (t3[k] - t2[k]) / 1e3, n_post[k] > 0
+    split = lambda x: f'{np.median(x):5.2f} / {x.max():5.2f} ({len(x):4d})' if len(x) else '    -         (   0)'
+    print(f'{k:6d} |             {attr(k, wa)} |            {attr(k, we)} | {split(post[m])} | {split(post[~m])}')
+k = slice(4, RING)
+post, m = (t3[k] - t2[k]) / 1e3, n_post[k] > 0
+print(f'launches 4..31: warps with an fp64 pass after the wait {m.mean():.2%} (links before / after the wait per launch: '
+      f'{n_pre[k].sum(1).mean():.1f} / {n_post[k].sum(1).mean():.1f}; overflow envs per launch {n_ovf[k].sum(1).mean():.1f})')
+print(f'  last warp to end ran a post-wait pass in {np.mean([n_post[j, t3[j].argmax()] > 0 for j in range(4, RING)]):.0%} of launches, '
+      f'an overflow env in {np.mean([n_ovf[j, t3[j].argmax()] > 0 for j in range(4, RING)]):.0%}; '
+      f'last warp at the wait: overflow env in {np.mean([n_ovf[j, t1[j].argmax()] > 0 for j in range(4, RING)]):.0%}')
+if m.any():
+    print(f'  release->end with a post-wait pass: median {np.median(post[m]):.2f} us, without: {np.median(post[~m]):.2f} us')
 np.save(Path(__file__).resolve().parent.parent / 'gpurun_out' / f'timeline_E{E}.npy', rec)
