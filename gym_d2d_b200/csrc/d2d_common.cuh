@@ -130,7 +130,7 @@ struct D2DParams {
 // Instrumented build only: every warp of the warp kernel stamps (globaltimer at entry, clock64 at entry / before
 // griddepcontrol.wait / after it / at its end, SM id) so that profiles/timeline.py can lay consecutive launches side by side,
 // and counts what the warp did: envs stepped, flagged links recomputed in fp64 before / after its wait, envs that took the
-// all-pairs overflow path.
+// overflow pass (an RB above D2D_BIN_CAP links).
 #define D2D_TL_SLOTS 64
 #define D2D_TL_WARPS 4096
 struct D2DTlRec { unsigned long long g0, c0, c1, c2, c3, smid, n_env, n_pre, n_post, n_ovf; };

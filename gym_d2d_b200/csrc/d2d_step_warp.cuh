@@ -20,8 +20,8 @@
 // after which a victim's co-channel peers are the first count[rb] records of ITS bin: no prefix scan, no offsets, no
 // scatter pass.  The first D2D_WALK_INLINE records are handled branch-free (immediate-offset LDS, predicated terms, so
 // the loads and gains of a lane's two victims overlap); fuller bins take a short serial loop.  An RB that holds more
-// than D2D_BIN_CAP links (~0.6 % of envs at the default load, but a policy may put every agent on one RB) sends the
-// env down an all-pairs shuffle path that needs no table at all - slower, same results.
+// than D2D_BIN_CAP links (~0.4 % of envs at the default load, but a policy may put every agent on one RB) keeps its
+// first D2D_BIN_CAP links in the bin; the links ranked beyond it add their terms in a shuffle pass over just those links.
 //
 // All CUE links share one receiver (the MBS at the origin), so there an interferer contributes a per-link scalar
 // u_k = w_k g(|tx_k|) computed once, and a CUE victim's walk is a sum of u_k; a DUE victim evaluates
@@ -326,22 +326,23 @@ __device__ __forceinline__ D2DLinkOut d2d_link_epilogue_warp(bool live, float p_
 
 // ---- rare paths -----------------------------------------------------------------------------------------------------------
 
-// Some RB holds more links than a bin has record slots: all-pairs pass over the 64 link slots by shuffle (no table).
-// A term counts when the RB keys match and it is not the victim itself.  Returns (I_A, I_B, dmin2_A, dmin2_B).
-// Only lanes with a live link are visited, in lane order: a lane whose two slots are both dead (inactive keys, unique per lane
-// and slot) matches no victim but itself, so every term it would add is exactly 0.0f and skipping it changes no bit.  In a late
-// launch this path is on the last warp to reach the wait in almost every launch of a one-wave batch (profiles/timeline.py).
+// Some RB holds more links than a bin has record slots: the links ranked D2D_BIN_CAP and above have no record, and this pass
+// adds their terms by shuffle (the bin walk has already added those of the records).  Source keys: the RB of a live slot of
+// rank >= D2D_BIN_CAP, the slot's unique inactive key otherwise; victim keys: the RB of every live slot.  A term counts when
+// the keys match and it is not the victim itself.  The terms go on top of the bin walk's sums IA / IB (and, with EXACT, its
+// distances dmin2A / dmin2B), in lane order.
+// Only lanes that hold such a source are visited, in lane order: at the default load one lane, rarely two (an RB of 9 or 10
+// links); with every link on one RB at most 25.  Any other lane matches no victim but itself, so skipping it changes no bit.
 #ifndef D2D_RARE_ATTR
 #define D2D_RARE_ATTR __forceinline__     // A/B knob: __noinline__ moves the rare paths out of the hot loop's code
 #endif
 template <bool PLE2, bool EXACT>
-__device__ D2D_RARE_ATTR float4 d2d_all_pairs_warp(uint32_t lane, uint32_t keyA, uint32_t keyB, float4 recA, float4 pB, float wB, float uB,
-                                                      float nhp) {
-    float IA = 0.f, IB = 0.f, dminA = 3.0e38f, dminB = 3.0e38f;
+__device__ D2D_RARE_ATTR void d2d_overflow_warp(uint32_t lane, uint32_t keyA, uint32_t keyB, uint32_t srcA, uint32_t srcB, float4 recA,
+                                                   float4 pB, float wB, float uB, float nhp, float &IA, float &IB, float &dminA, float &dminB) {
 #pragma unroll 1
-    for (uint32_t src = __ballot_sync(0xffffffffu, (keyA & keyB & D2D_INACTIVE_KEY) == 0u); src; src &= src - 1u) {
+    for (uint32_t src = __ballot_sync(0xffffffffu, (srcA & srcB & D2D_INACTIVE_KEY) == 0u); src; src &= src - 1u) {
         const uint32_t k = (uint32_t)__ffs((int)src) - 1u;
-        const uint32_t kA = __shfl_sync(0xffffffffu, keyA, k), kB = __shfl_sync(0xffffffffu, keyB, k);
+        const uint32_t kA = __shfl_sync(0xffffffffu, srcA, k), kB = __shfl_sync(0xffffffffu, srcB, k);
         const float4 ra = make_float4(__shfl_sync(0xffffffffu, recA.x, k), __shfl_sync(0xffffffffu, recA.y, k),
                                       __shfl_sync(0xffffffffu, recA.z, k), __shfl_sync(0xffffffffu, recA.w, k));
         const float4 rb = make_float4(__shfl_sync(0xffffffffu, pB.x, k), __shfl_sync(0xffffffffu, pB.y, k),
@@ -356,7 +357,6 @@ __device__ D2D_RARE_ATTR float4 d2d_all_pairs_warp(uint32_t lane, uint32_t keyA,
         IB += d2d_term_rx<PLE2, EXACT>(ra, kA == keyB, pB.z, pB.w, nhp, dminB);
         IB += d2d_term_rx<PLE2, EXACT>(rb, kB == keyB && k != lane, pB.z, pB.w, nhp, dminB);
     }
-    return make_float4(IA, IB, dminA, dminB);
 }
 
 __device__ __forceinline__ double d2d_shfl_f64(double v, int src) {
@@ -660,21 +660,23 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
         // ---- simulator.py:95-101: interference at each victim's receiver (a dead lane has an empty range) ----------
         const uint2 ctA = d2d_lds64u_at<0>(cntA);                              // (links on the victim's RB, SIDELINK flag)
         const uint32_t nA = ctA.x, nB = d2d_lds32u_at<0>(cntB);
-        float IA, IB, dminA = 3.0e38f, dminB = 3.0e38f;
-        if (__any_sync(0xffffffffu, (liveA && nA > D2D_BIN_CAP) || (liveB && nB > D2D_BIN_CAP))) {
-            // rare: some RB holds more links than a bin has record slots
+        float dminA = 3.0e38f, dminB = 3.0e38f;
+        // bit t of valid <=> record t of the victim's bin exists and is not the victim (dead lane: 0).  An RB of more than
+        // D2D_BIN_CAP links has D2D_BIN_CAP records; a victim ranked beyond them has none to exclude.
+        const uint32_t validA = liveA ? (((1u << min(nA, (uint32_t)D2D_BIN_CAP)) - 1u) & ~(rankA < D2D_BIN_CAP ? 1u << rankA : 0u)) : 0u;
+        const uint32_t validB = liveB ? (((1u << min(nB, (uint32_t)D2D_BIN_CAP)) - 1u) & ~(rankB < D2D_BIN_CAP ? 1u << rankB : 0u)) : 0u;
+        float IA = EXACT ? d2d_walk_rx<PLE2, true>(binA, zrec, validA, 0.f, 0.f, P.neg_half_ple, dminA) : d2d_walk_mbs(binA, zrec, validA);
+        float IB = d2d_walk_rx<PLE2, EXACT>(binB, zrec, validB, pB.z, pB.w, P.neg_half_ple, dminB);
+        const bool ovfA = liveA && rankA >= D2D_BIN_CAP, ovfB = liveB && rankB >= D2D_BIN_CAP;
+        if (__any_sync(0xffffffffu, ovfA || ovfB)) {
+            // rare: some RB holds more links than a bin has record slots - add the links without a record
             const uint32_t keyA = liveA ? rbA : (D2D_INACTIVE_KEY | lane), keyB = liveB ? rbB : (D2D_INACTIVE_KEY | 32u | lane);
-            const float4 r = d2d_all_pairs_warp<PLE2, EXACT>(lane, keyA, keyB, make_float4(tA.x, tA.y, wA, uA), pB, wB, uB, P.neg_half_ple);
-            IA = r.x; IB = r.y; dminA = r.z; dminB = r.w;
+            const uint32_t srcA = ovfA ? rbA : (D2D_INACTIVE_KEY | lane), srcB = ovfB ? rbB : (D2D_INACTIVE_KEY | 32u | lane);
+            d2d_overflow_warp<PLE2, EXACT>(lane, keyA, keyB, srcA, srcB, make_float4(tA.x, tA.y, wA, uA), pB, wB, uB, P.neg_half_ple,
+                                           IA, IB, dminA, dminB);
 #ifdef D2D_TIMELINE
             ++tl_ovf;
 #endif
-        } else {
-            // bit t of valid <=> record t of the victim's bin exists and is not the victim (dead lane: 0)
-            const uint32_t validA = liveA ? (((1u << nA) - 1u) ^ (1u << rankA)) : 0u;
-            const uint32_t validB = liveB ? (((1u << nB) - 1u) ^ (1u << rankB)) : 0u;
-            IA = EXACT ? d2d_walk_rx<PLE2, true>(binA, zrec, validA, 0.f, 0.f, P.neg_half_ple, dminA) : d2d_walk_mbs(binA, zrec, validA);
-            IB = d2d_walk_rx<PLE2, EXACT>(binB, zrec, validB, pB.z, pB.w, P.neg_half_ple, dminB);
         }
 
         // ---- per-link epilogue (simulator.py:93,106-107,110-127,144-154); dead lanes are zeroed ------------------------

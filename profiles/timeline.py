@@ -5,8 +5,9 @@ globaltimer + clock64 at entry, clock64 before / after griddepcontrol.wait and a
 a CUDA graph of 32 step launches (the bench's launch mode), reads the stamps of the last replay and prints, per launch, when
 its warps started / reached the wait / were released / ended - relative to the previous launch - i.e. how much of a step
 overlaps its predecessor under programmatic dependent launch.  Every warp also counts the envs it stepped, the flagged links it
-recomputed in fp64 before / after its wait and the envs that took the all-pairs overflow path; the script prints them for the
-last warp to reach the wait and the last to end, and splits the post-wait time by whether a warp ran an fp64 pass after its wait.
+recomputed in fp64 before / after its wait and the envs that took the overflow pass (an RB above D2D_BIN_CAP links); the script
+prints them for the last warp to reach the wait and the last to end, splits the post-wait time by whether a warp ran an fp64 pass
+after its wait, and the entry -> wait time by whether it stepped an overflow env.
 Numbers from an instrumented build are not bench values.
 """
 import ctypes
@@ -109,4 +110,13 @@ print(f'  last warp to end ran a post-wait pass in {np.mean([n_post[j, t3[j].arg
       f'last warp at the wait: overflow env in {np.mean([n_ovf[j, t1[j].argmax()] > 0 for j in range(4, RING)]):.0%}')
 if m.any():
     print(f'  release->end with a post-wait pass: median {np.median(post[m]):.2f} us, without: {np.median(post[~m]):.2f} us')
+# entry -> wait of the warps that stepped an env with an RB above D2D_BIN_CAP links, against the others
+pre, o = (t1[k] - t0[k]) / 1e3, n_ovf[k] > 0
+split = lambda x: f'median {np.median(x):5.2f} us  max {x.max():5.2f} us ({x.size} warps)' if x.size else '-'
+print(f'  entry->wait with an overflow env: {split(pre[o])}; without: {split(pre[~o])}')
+wa = [int(t1[j].argmax()) for j in range(4, RING)]
+print(f'  last warp at the wait, launches 4..31: envs {np.mean([n_env[j, w] for j, w in zip(range(4, RING), wa)]):.1f}, '
+      f'fp64 links before / after the wait {np.mean([n_pre[j, w] for j, w in zip(range(4, RING), wa)]):.2f} / '
+      f'{np.mean([n_post[j, w] for j, w in zip(range(4, RING), wa)]):.2f}, '
+      f'overflow env in {np.mean([n_ovf[j, w] > 0 for j, w in zip(range(4, RING), wa)]):.0%}')
 np.save(Path(__file__).resolve().parent.parent / 'gpurun_out' / f'timeline_E{E}.npy', rec)
