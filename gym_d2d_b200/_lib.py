@@ -49,6 +49,7 @@ class D2DStepIO(C.Structure):
 
 STEP_INPUTS_STABLE = 1          # d2d_step_io.flags (include/d2d_b200.h, "Ordering rule")
 STEP_ACTIONS_I16 = 2            # d2d_step_host*: `actions` is int16 [E][N]
+STEP_AUTORESET = 4              # d2d_step: next-step auto-reset of envs whose previous step returned done
 EPISODE_DRAW_ACTIONS = 1        # d2d_episode flags
 OUT_OBS, OUT_CAPACITY, OUT_REWARD, OUT_DONE, OUT_RATE, OUT_RB, OUT_TX_PWR, OUT_AGENT_REWARD, OUT_OBS_DYN = (
     1, 2, 4, 8, 16, 32, 64, 128, 256)
@@ -72,6 +73,7 @@ SIGNATURES = {
     'd2d_state_bytes': (C.c_int, [_vp, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
     'd2d_bind_state': (C.c_int, [_vp, _vp, _vp, _vp]),
     'd2d_bind_positions_f64': (C.c_int, [_vp, _vp]),
+    'd2d_bind_autoreset': (C.c_int, [_vp, _vp, _u64]),
     'd2d_set_positions': (C.c_int, [_vp, _vp, C.c_int, _i64, _i64, _vp]),
     'd2d_reset': (C.c_int, [_vp, _u64, _u64, _vp, _vp]),
     'd2d_get_positions': (C.c_int, [_vp, _vp, C.c_int, _i64, _i64, _vp]),

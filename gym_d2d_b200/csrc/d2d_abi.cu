@@ -75,6 +75,7 @@ D2DParams make_params(const d2d_handle *h, const d2d_step_io_t *io) {
     P.ple_d = h->ple;
     P.linkA = h->dA; P.linkB = h->dB; P.linkD = h->dD; P.link_meta = h->dMeta; P.pwr_lin = h->dPwr; P.pwr_lin_d = h->dPwrD;
     P.pos = h->pos; P.pos64 = h->pos64; P.step_count = h->step_count; P.stats = h->stats;
+    P.episode_index = h->episode_index; P.ar_base = h->ar_base;
     P.rng_step_dev = h->dRngStep;
     P.cell_radius = (float)h->cfg.cell_radius_m; P.d2d_radius = (float)h->cfg.d2d_radius_m;
     P.pos_out = h->pos;
@@ -373,6 +374,16 @@ D2D_API int d2d_bind_positions_f64(d2d_handle_t *h, double *positions_f64) {
     return D2D_OK;
 }
 
+D2D_API int d2d_bind_autoreset(d2d_handle_t *h, uint32_t *episode_index, uint64_t base_key) {
+    if (!h) return fail(D2D_ERR_INVALID_ARG, "d2d_bind_autoreset: null handle");
+    if (episode_index && !h->use_warp)
+        return fail(D2D_ERR_UNSUPPORTED, "d2d_bind_autoreset: auto-reset runs on the warp kernel only (<= 32 CUEs, <= 32 DUE pairs, <= 64 RBs, "
+                                         "no downlinks, no ShadowingPathLoss)");
+    h->episode_index = episode_index;
+    h->ar_base = base_key;
+    return D2D_OK;
+}
+
 D2D_API int d2d_set_positions(d2d_handle_t *h, const double *src, int src_on_device, int64_t first_env, int64_t count,
                               void *stream) {
     if (!h || !src) return fail(D2D_ERR_INVALID_ARG, "d2d_set_positions: null argument");
@@ -479,8 +490,9 @@ namespace {
 enum { MODE_STEP = 0, MODE_MANY = 1, MODE_EPISODE = 2 };
 
 // per-agent rewards (SHANNON / CUE_SINR_SHANNON always; SYSTEM_CAPACITY when the caller asked for the broadcast): one more
-// small kernel over `total` env-steps of io; `with_stats`: the reward statistics of the per-agent functions
-int agent_reward_launch(d2d_handle *h, const d2d_step_io_t *io, int64_t total, bool with_stats, cudaStream_t st) {
+// small kernel over `total` env-steps of io; `with_stats`: the reward statistics of the per-agent functions; `autoreset`: rows
+// whose step counter is 0 after the step were reset by it (D2D_STEP_AUTORESET) and score nothing
+int agent_reward_launch(d2d_handle *h, const d2d_step_io_t *io, int64_t total, bool with_stats, cudaStream_t st, bool autoreset = false) {
     if (!io->obs || !io->reward || !io->actions) return fail(D2D_ERR_INVALID_ARG, "per-agent rewards need the actions, obs and reward buffers");
     const bool warp_team = h->N <= 64;
     const int teams = warp_team ? 8 : 1;
@@ -488,12 +500,13 @@ int agent_reward_launch(d2d_handle *h, const d2d_step_io_t *io, int64_t total, b
     // only CueSinrShannon keeps per-RB counters in shared memory (opt-in done by d2d_create)
     const size_t smem = h->cfg.reward_fn == D2D_REWARD_CUE_SINR_SHANNON ? (size_t)teams * h->cfg.num_rbs * sizeof(uint32_t) : 0;
     double *stats = with_stats && h->cfg.reward_fn != D2D_REWARD_SYSTEM_CAPACITY ? h->stats : nullptr;
+    const uint8_t *counters = autoreset ? h->step_count : nullptr;
     if (warp_team)
         d2d_agent_reward_kernel<32><<<grid, 256, smem, st>>>(io->actions, io->obs, io->agent_reward, io->reward, stats, total, h->N,
-                                                            h->dMeta, h->cfg.num_rbs, h->cfg.reward_fn, (float)h->cfg.reward_param);
+                                                            h->dMeta, h->cfg.num_rbs, h->cfg.reward_fn, (float)h->cfg.reward_param, counters);
     else
         d2d_agent_reward_kernel<256><<<grid, 256, smem, st>>>(io->actions, io->obs, io->agent_reward, io->reward, stats, total, h->N,
-                                                             h->dMeta, h->cfg.num_rbs, h->cfg.reward_fn, (float)h->cfg.reward_param);
+                                                             h->dMeta, h->cfg.num_rbs, h->cfg.reward_fn, (float)h->cfg.reward_param, counters);
     D2D_CUDA(cudaGetLastError());
     ++h->launches;
     return D2D_OK;
@@ -516,6 +529,8 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
     const bool draw_actions = ea.draw_actions;
     cudaStream_t st = (cudaStream_t)stream;
     const bool many = mode != MODE_STEP;
+    // D2D_STEP_AUTORESET (d2d_step only): always the default ordering - wait at entry, no late wait, no tickets, the full grid
+    const bool autoreset = mode == MODE_STEP && (io->flags & D2D_STEP_AUTORESET) != 0u;
     // "Ordering rule" of include/d2d_b200.h: inputs may be read ahead of griddepcontrol.wait only on the caller's promise AND when
     // the kernel before this one (for this handle, in this stream) was a step kernel, which writes neither actions nor positions.
     // An episode that draws its own actions reads no input at all.
@@ -524,7 +539,7 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
     const bool reads_positions = mode != MODE_EPISODE || ea.no_reset;
     if (!reads_positions && draw_actions) stable = h->pdl;
     else if (!reads_positions) stable = stable && (io->flags & D2D_STEP_INPUTS_STABLE) && h->last_kind != D2D_LAST_OTHER;
-    else stable = stable && (io->flags & D2D_STEP_INPUTS_STABLE) && h->last_kind == D2D_LAST_STEP;
+    else stable = stable && (io->flags & D2D_STEP_INPUTS_STABLE) && h->last_kind == D2D_LAST_STEP && !autoreset;
     P.flags = (stable ? 0u : D2D_PF_INPUTS_FRESH) | (draw_actions ? D2D_PF_DRAW_ACTIONS : 0u) | (ea.no_reset ? D2D_PF_NO_RESET : 0u);
     // Late wait (d2d_step_warp.cuh): a flagged single-launch d2d_step right behind another one of this handle, whose per-link output
     // buffers alias none of the previous step's, stores them ahead of griddepcontrol.wait - nothing the predecessor does can
@@ -539,7 +554,7 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
         const size_t EN = (size_t)h->cfg.num_envs * h->N;
         const uintptr_t cur[6][2] = {{(uintptr_t)io->obs, EN * 24}, {(uintptr_t)io->obs_dyn, EN * 8}, {(uintptr_t)io->capacity_mbps, EN * 4},
                                      {(uintptr_t)io->rate_bps, EN * 4}, {(uintptr_t)io->rb, EN * 2}, {(uintptr_t)io->tx_pwr_dBm, EN * 2}};
-        const bool plain = h->use_warp && mode == MODE_STEP && h->cfg.reward_fn == D2D_REWARD_SYSTEM_CAPACITY && !io->agent_reward && !h->dRngStep &&
+        const bool plain = h->use_warp && mode == MODE_STEP && !autoreset && h->cfg.reward_fn == D2D_REWARD_SYSTEM_CAPACITY && !io->agent_reward && !h->dRngStep &&
                            h->cfg.num_envs <= std::max<int64_t>(1, (int64_t)0x7fffffff / std::max(6 * h->N, 2 * h->V)) &&
                            !(h->chunk_override > 0 && h->chunk_override < h->cfg.num_envs);
         late = plain && stable && h->late_wait_on && h->prev_out_valid && h->last_kind == D2D_LAST_STEP && !(h->wpb == 2 && h->cfg.num_envs > 1792 && h->grid_late == 0);
@@ -554,13 +569,13 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
     // geometry, inputs declared stable - waits per warp for that token instead of for the whole grid.
     // (not when a post-pass kernel follows the step kernel: the next step's predecessor in the stream is then that kernel; and only
     // for steps that write buffers their predecessor wrote - the late wait above serves the others)
-    const bool single_launch = !late && h->use_warp && mode == MODE_STEP && h->dTickets && h->pdl && h->tickets_on &&
+    const bool single_launch = !late && h->use_warp && mode == MODE_STEP && !autoreset && h->dTickets && h->pdl && h->tickets_on &&
                                h->cfg.reward_fn == D2D_REWARD_SYSTEM_CAPACITY && !io->agent_reward && !h->dRngStep &&
                                h->cfg.num_envs <= std::max<int64_t>(1, (int64_t)0x7fffffff / std::max(6 * h->N, 2 * h->V)) &&
                                !(h->chunk_override > 0 && h->chunk_override < h->cfg.num_envs);
     // (late: one chunk, never a fused launch; grid_fresh: an A/B knob, 0 by default - see d2d_create)
     const int step_grid = late && h->grid_late > 0 ? std::min(h->grid, h->grid_late)
-                          : (!stable && mode == MODE_STEP && h->grid_fresh > 0) ? std::min(h->grid, h->grid_fresh) : h->grid;
+                          : (!stable && mode == MODE_STEP && !autoreset && h->grid_fresh > 0) ? std::min(h->grid, h->grid_fresh) : h->grid;
     const int grid1 = (int)std::min<int64_t>(step_grid, (h->cfg.num_envs + h->envs_per_block - 1) / h->envs_per_block);
     // measured (profiles/README.md): the per-warp hand-off wins as soon as warps step more than one env per launch (E = 6 144,
     // 1.5 envs per warp: 7.6 -> 5.3 us; E = 16 384: 12.4 -> 9.4 us; E = 131 072: 69.5 -> 65.9 us) and loses at exactly one
@@ -590,6 +605,7 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
             P.pos += chunk * h->V * 2; P.pos_out += chunk * h->V * 2;
             if (P.pos64) P.pos64 += chunk * h->V * 2;
             if (P.step_count) P.step_count += chunk;
+            if (P.episode_index) P.episode_index += chunk;
             if (P.obs) P.obs += dl * 6;
             if (P.obs_dyn) P.obs_dyn += dl;
             if (P.cap) P.cap += dl;
@@ -612,6 +628,7 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
         D2DLaunchSel sel;
         sel.many = mode == MODE_MANY; sel.episode = mode == MODE_EPISODE;
         sel.no_reset = ea.no_reset;
+        sel.autoreset = autoreset;
         sel.fast = mode == MODE_EPISODE && draw_actions && !io->actions_out;
         sel.exact = h->pos64 != nullptr;
         sel.smem = alt ? h->many.smem : h->smem;
@@ -628,18 +645,25 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
     }
     D2D_CUDA(cudaGetLastError());
     h->last_stream = stream;
-    h->last_kind = mode == MODE_EPISODE && !ea.no_reset ? D2D_LAST_EPISODE : D2D_LAST_STEP;
+    // (an auto-reset step wrote positions: the next step reads them after its wait, as after an episode)
+    h->last_kind = (mode == MODE_EPISODE && !ea.no_reset) || autoreset ? D2D_LAST_EPISODE : D2D_LAST_STEP;
     if (h->dRngStep) {      // ShadowingPathLoss: the next call draws fresh values, also when this one is replayed from a CUDA graph
         d2d_advance_counter_kernel<<<1, 1, 0, st>>>(h->dRngStep, (uint64_t)T);
         D2D_CUDA(cudaGetLastError());
     }
     if (mode != MODE_EPISODE && (h->cfg.reward_fn != D2D_REWARD_SYSTEM_CAPACITY || io->agent_reward))
-        return agent_reward_launch(h, io, (int64_t)T * h->cfg.num_envs, true, st);
+        return agent_reward_launch(h, io, (int64_t)T * h->cfg.num_envs, true, st, autoreset);
     return D2D_OK;
 }
 
-int check_step_args(const d2d_handle_t *h, const d2d_step_io_t *io, const char *who, bool need_actions = true) {
+int check_step_args(const d2d_handle_t *h, const d2d_step_io_t *io, const char *who, bool need_actions = true, bool autoreset_ok = false) {
     if (!h || !io || (need_actions && !io->actions)) return fail(D2D_ERR_INVALID_ARG, std::string(who) + ": handle, io and io->actions are required");
+    if (io->flags & D2D_STEP_AUTORESET) {
+        if (!autoreset_ok || !h->use_warp)
+            return fail(D2D_ERR_UNSUPPORTED, std::string(who) + ": D2D_STEP_AUTORESET applies to d2d_step on warp-kernel configurations only");
+        if (!h->episode_index || !h->step_count)
+            return fail(D2D_ERR_STATE, std::string(who) + ": D2D_STEP_AUTORESET needs d2d_bind_autoreset and a bound step counter");
+    }
     if (!h->pos) return fail(D2D_ERR_STATE, std::string(who) + ": call d2d_bind_state first");
     if (io->flags & D2D_STEP_ACTIONS_I16)      // (d2d_step_host_async clears the flag on the device-side io it passes down)
         return fail(D2D_ERR_INVALID_ARG, std::string(who) + ": D2D_STEP_ACTIONS_I16 applies to d2d_step_host / d2d_step_host_async only");
@@ -667,7 +691,7 @@ void advance_io(d2d_step_io_t &cur, int64_t steps, int64_t E, int N) {
 }  // namespace
 
 D2D_API int d2d_step(d2d_handle_t *h, const d2d_step_io_t *io, void *stream) {
-    int rc = check_step_args(h, io, "d2d_step");
+    int rc = check_step_args(h, io, "d2d_step", true, true);
     if (rc) return rc;
     D2D_GUARD(h);
     return step_launch(h, io, 1, MODE_STEP, stream);
@@ -881,6 +905,7 @@ D2D_API int d2d_host_slot_buffers(d2d_handle_t *h, int slot, uint32_t outputs, d
 D2D_API int d2d_step_host_async(d2d_handle_t *h, const d2d_step_io_t *hio, int slot, void *stream) {
     if (!h || !hio || !hio->actions) return fail(D2D_ERR_INVALID_ARG, "d2d_step_host_async: handle, io and io->actions are required");
     if (slot < 0 || slot >= D2D_HOST_SLOTS) return fail(D2D_ERR_INVALID_ARG, "d2d_step_host_async: slot must be in [0, D2D_HOST_SLOTS)");
+    if (hio->flags & D2D_STEP_AUTORESET) return fail(D2D_ERR_UNSUPPORTED, "d2d_step_host_async: D2D_STEP_AUTORESET applies to d2d_step only");
     if (!h->pos) return fail(D2D_ERR_STATE, "d2d_step_host_async: call d2d_bind_state first");
     D2D_GUARD(h);
     int rc = host_pipeline_init(h);

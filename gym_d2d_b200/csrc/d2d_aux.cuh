@@ -117,10 +117,13 @@ __global__ void d2d_per_agent_obs_kernel(const float *__restrict__ table, float 
 // Reads the decoded step results (sinr_dB from the observation table - after the fp64 pass, so threshold decisions see the
 // rescued values) and re-derives the RB from the raw action (envs/d2d_env.py:93-101).  For modes 1 / 2 reward[e] becomes
 // the mean agent reward and the reward statistics are accumulated here (the step kernel skips them).
+// reset_rows (D2D_STEP_AUTORESET, else NULL): the step counters after the step.  A row at 0 was reset by the step, whose actions are
+// not the caller's: it has no acting agent - agent_reward 0, reward 0, nothing added to the statistics.
 template <int TEAM>
 __global__ void d2d_agent_reward_kernel(const int32_t *__restrict__ actions, const float *__restrict__ obs,
                                         float *__restrict__ agent_reward, float *__restrict__ reward, double *__restrict__ stats,
-                                        int64_t num_envs, int N, const int32_t *__restrict__ link_meta, int R, int mode, float param) {
+                                        int64_t num_envs, int N, const int32_t *__restrict__ link_meta, int R, int mode, float param,
+                                        const uint8_t *__restrict__ reset_rows) {
     extern __shared__ uint32_t d2d_weak_smem[];
     const int teams = blockDim.x / TEAM, team = threadIdx.x / TEAM, tl = threadIdx.x % TEAM;
     uint32_t *weak = d2d_weak_smem + (size_t)team * R;         // mode 2 only (the launch requests no shared memory otherwise)
@@ -130,12 +133,13 @@ __global__ void d2d_agent_reward_kernel(const int32_t *__restrict__ actions, con
     for (int64_t it = 0; it < rounds; ++it) {
         const int64_t e = (it * gridDim.x + blockIdx.x) * teams + team;
         const bool in = e < num_envs;                 // whole teams drop out together; barriers stay uniform per block
+        const bool acts = in && !(reset_rows && reset_rows[e] == 0);
         const int32_t *act = actions + (in ? e : 0) * N;
         const float *ob = obs + (in ? e : 0) * N * 6;
         if (mode == 2) {
             for (int r = tl; r < R; r += TEAM) weak[r] = 0u;
             team_sync();
-            for (int j = tl; in && j < N; j += TEAM) {
+            for (int j = tl; acts && j < N; j += TEAM) {
                 const int meta = link_meta[j], npw = meta & 0xffff;          // power levels | SIDELINK << 16
                 const uint32_t a = (uint32_t)act[j];
                 if (!(meta >> 16) && a < (uint32_t)(R * npw) && ob[j * 6 + 4] < param) atomicAdd(&weak[a / (uint32_t)npw], 1u);
@@ -147,7 +151,7 @@ __global__ void d2d_agent_reward_kernel(const int32_t *__restrict__ actions, con
         for (int j = tl; in && j < N; j += TEAM) {
             const int meta = link_meta[j], npw = meta & 0xffff;
             const uint32_t a = (uint32_t)act[j];
-            const bool live = a < (uint32_t)(R * npw);
+            const bool live = acts && a < (uint32_t)(R * npw);
             float rw = 0.f;
             if (live) {
                 const float sinr = ob[j * 6 + 4];

@@ -124,6 +124,9 @@ struct D2DParams {
 #ifdef D2D_TIMELINE
     int32_t tl_slot;             // instrumented build (profiles/timeline.py): which d2d_tl_buf slot this launch stamps
 #endif
+    // d2d_step with D2D_STEP_AUTORESET (warp kernel, MODE 5).  Last in the struct, so every other kernel's parameter offsets stay put.
+    uint32_t *episode_index;     // [E] episodes each env has begun since the last full reset (caller-owned)
+    uint64_t ar_base;            // base of the per-env reset keys: env e's n-th auto-reset draws under d2d_autoreset_key(ar_base, n)
 };
 
 #ifdef D2D_TIMELINE
@@ -289,6 +292,16 @@ __device__ __forceinline__ uint4 d2d_action_block(uint64_t act_seed, uint64_t ge
 }
 __device__ __forceinline__ uint32_t d2d_action_word(const uint4 &b, uint32_t t, bool due) {
     return (t & 1u) ? (due ? b.w : b.z) : (due ? b.y : b.x);
+}
+
+// Auto-reset (D2D_STEP_AUTORESET): the Philox key of an env's n-th episode since the last full reset, key(base, n) =
+// splitmix64(base + n * 0x9E3779B97F4A7C15) with splitmix64 the output function of Steele et al.'s SplitMix64.  Philox's counter
+// carries the global env, so the draws depend on (base, global env, n) only.  Mirrored by VecD2DEnv.autoreset_key.
+__host__ __device__ __forceinline__ uint64_t d2d_autoreset_key(uint64_t base, uint64_t n) {
+    uint64_t z = base + n * 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
 }
 
 // The N(0,1) draw of one ShadowingPathLoss evaluation (kind 0: the terms of the SINR, 1: the SNR's own-link evaluation): Box-Muller

@@ -73,6 +73,8 @@ struct d2d_handle {
     double *pos64 = nullptr;
     uint8_t *step_count = nullptr;
     double *stats = nullptr;
+    uint32_t *episode_index = nullptr;   // d2d_bind_autoreset
+    uint64_t ar_base = 0;
     // host-buffer steps (d2d_step_host*): the pipeline slots
     d2d_host_slot slot[D2D_HOST_SLOTS];
     cudaStream_t s_in = nullptr, s_out = nullptr, s_out2 = nullptr;      // s_out2: odd slots' copy-out (D2D_B200_OUT_STREAMS=2, A/B)
@@ -180,6 +182,7 @@ struct D2DLaunchSel {
     bool episode = false;    // d2d_episode / d2d_rollout: P.T slices per env; positions and / or actions are drawn inside the kernel
     bool fast = false;       // ... with drawn actions, no action record and no fp64 shadow: the compiled-in variants
     bool no_reset = false;   // ... d2d_rollout
+    bool autoreset = false;  // d2d_step with D2D_STEP_AUTORESET (warp kernel only)
     int smem = 0;            // dynamic shared memory of the geometry this launch uses
 };
 

@@ -381,14 +381,16 @@ __device__ __forceinline__ double d2d_shfl_xor_f64(double v, int m) {
 // Without a position shadow a dB value is rewritten only when its linear ratio is within 1/16 of one - the only place the
 // fp32 value is ill-conditioned; rate and capacity are well conditioned there and are rewritten only if the sensitivity
 // gate (simulator.py:123,149) could sit inside that band.  With a shadow every output of the link is rewritten.
+// AR (d2d_step with auto-reset): `drawn` marks an env whose positions this launch drew; the shadow rows still hold the finished
+// episode's, so the pass takes the lane's fp32 registers - the values the launch stores to the shadow.
 // Returns the number of links recomputed.
 // 10^(p/10) in fp64 for the warp kernel's fp64 pass: the constant bank instead of a global table (filled by d2d_create)
 static __constant__ double d2d_pwr_lin_c[D2D_MAX_PWR_LEVELS];    // one copy per translation unit (d2d_tu_warp.cu)
 
-template <bool PLE2, bool EXACT, bool SPEC, bool STORE, bool THR>
+template <bool PLE2, bool EXACT, bool SPEC, bool STORE, bool THR, bool AR = false>
 __device__ __forceinline__ int d2d_rescue_warp(const D2DParams &P, const D2DShape<SPEC> &S, uint32_t e, uint32_t lane, uint32_t jA,
                                                uint32_t keyA, uint32_t keyB, bool needA, bool needB, uint32_t pA, uint32_t pB_,
-                                               const float2 &tA, const float4 &pB, D2DLinkOut &oA, D2DLinkOut &oB) {
+                                               const float2 &tA, const float4 &pB, D2DLinkOut &oA, D2DLinkOut &oB, bool drawn = false) {
     const uint32_t C = S.C(), V = S.V();
     // Without an fp64 shadow the positions ARE the fp32 state the lane already holds; with uniform link constants (one set per
     // link type: every default-shape batch) those come from the constant bank, like the power table: then the pass reads
@@ -397,7 +399,7 @@ __device__ __forceinline__ int d2d_rescue_warp(const D2DParams &P, const D2DShap
     // this lane's two transmitters and the DUE receiver, in fp64
     double2 txA = make_double2((double)tA.x, (double)tA.y), txB = make_double2((double)pB.x, (double)pB.y);
     double2 rxB = make_double2((double)pB.z, (double)pB.w);
-    if (EXACT) {
+    if (EXACT && !(AR && drawn)) {
         const double2 *pe64 = reinterpret_cast<const double2 *>(P.pos64) + (int64_t)e * V;
         if (lane < C) txA = pe64[1u + lane];
         if (lane < S.D()) { txB = pe64[1u + C + 2u * lane]; rxB = pe64[2u + C + 2u * lane]; }
@@ -465,12 +467,12 @@ __device__ __forceinline__ int d2d_rescue_warp(const D2DParams &P, const D2DShap
 }
 
 // the throughput shapes' call of the pass (after the stores): one place to take it out of line
-template <bool PLE2, bool EXACT, bool SPEC, bool THR>
+template <bool PLE2, bool EXACT, bool SPEC, bool THR, bool AR = false>
 __device__ D2D_RARE_ATTR int d2d_rescue_warp_late(const D2DParams &P, const D2DShape<SPEC> &S, uint32_t e, uint32_t lane, uint32_t jA,
                                                   uint32_t keyA, uint32_t keyB, bool needA, bool needB, uint32_t pA, uint32_t pB_,
-                                                  float2 tA, float4 pB) {
+                                                  float2 tA, float4 pB, bool drawn = false) {
     D2DLinkOut oA, oB;       // unused by the storing variant
-    return d2d_rescue_warp<PLE2, EXACT, SPEC, true, THR>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_, tA, pB, oA, oB);
+    return d2d_rescue_warp<PLE2, EXACT, SPEC, true, THR, AR>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_, tA, pB, oA, oB, drawn);
 }
 
 // FULL: the caller passed exactly the core outputs (obs, capacity, reward, done) and a step counter is bound - the
@@ -486,11 +488,18 @@ __device__ D2D_RARE_ATTR int d2d_rescue_warp_late(const D2DParams &P, const D2DS
 // but its constant tables.  MODE 2 reads its variant from P.flags (given or drawn actions, d2d_episode or d2d_rollout, any
 // set of outputs); MODE 3 (episode) and MODE 4 (rollout) are the instantiations of the common case - drawn actions, exactly
 // the core outputs (FULL) - with those choices compiled in: 490 instead of 590 warp-instructions per env-step.
+// MODE 5 (AR): d2d_step with D2D_STEP_AUTORESET.  An env whose step counter is below episode_length at entry steps exactly as in
+// MODE 0; one at or past it (its previous step returned done) is reset instead, as D2DEnv.reset does it (envs/d2d_env.py:45-52):
+// positions drawn like d2d_reset and actions like d2d_sample_actions(step 0), both under d2d_autoreset_key(ar_base, n) with n its
+// incremented episode index, then one uncounted step on them.  Its outputs are that step's with reward = done = 0; its counter
+// becomes 0, the drawn positions the bound state.  The launch always waits at entry (the host never flags it INPUTS_STABLE or
+// LATE_WAIT), so each group's counters and episode indices are read into lanes before the group's first env is computed.
 template <bool PLE2, bool EXACT, int WPB, bool FULL, bool SPEC, int MODE>
 __global__ void __launch_bounds__(WPB * 32, D2D_WARP_MIN_BLOCKS(WPB))
 d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
     extern __shared__ __align__(16) unsigned char d2d_warp_smem[];
-    constexpr bool MANY = MODE != 0, EPI = MODE >= 2, EPI_FAST = MODE >= 3;
+    constexpr bool AR = MODE == 5;
+    constexpr bool MANY = MODE != 0 && !AR, EPI = MODE >= 2 && !AR, EPI_FAST = MODE == 3 || MODE == 4;
     static_assert(!EPI_FAST || FULL, "the fast episode / rollout instantiations write exactly the core outputs");
     const D2DShape<SPEC> S(P);
     // latency shape: the fp64 pass runs before griddepcontrol.wait
@@ -574,6 +583,9 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
     uint32_t g = 0;                                                // position of env e in its group of 32
     int ns_keep = 0;                                               // lane i: step counter of the group's env i
     float rew_keep = 0.f;                                          // lane i: reward of the group's env i
+    uint32_t ep_keep = 0;                                          // AR, lane i: episode index of the group's env i ...
+    bool rs_keep = false;                                          // ... and whether this launch resets it
+    uint32_t st_steps = 0;                                         // AR: counted env-steps of this warp
     // d2d_step_many state: step index inside the env, the link / env offsets of output slice t, the env's positions
     uint32_t t = 0, tN = 0, tE = 0;
     const uint32_t T = MANY ? (uint32_t)P.T : 1u, strideE = MANY ? (uint32_t)P.t_stride : 0u, strideN = strideE * N;
@@ -612,6 +624,25 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
                 aB = hasB ? __umulhi(d2d_action_word(ablk, ts, true), limB) : 0xffffffffu;
             }
         } else if (!MANY || t == 0u) { tA_keep = nxt.tA; pB_keep = nxt.pB; }
+        // AR: this env is reset instead of stepped.  Every use below reads (AR && ar_rst): a bare runtime flag, although constant
+        // false in the other modes, changed their instruction schedule
+        bool ar_rst = false;
+        if constexpr (AR) {
+            if (g == 0u) {
+                ns_keep = e + lane < e_end ? (int)P.step_count[e + lane] : 0;
+                ep_keep = e + lane < e_end ? P.episode_index[e + lane] : 0u;
+            }
+            ar_rst = __shfl_sync(0xffffffffu, ns_keep, (int)g) >= P.episode_length;
+            if (ar_rst) {                                           // (the prefetched positions and actions of this env go unused)
+                const uint64_t genv = P.first_global_env + (uint64_t)e;
+                const uint64_t key = d2d_autoreset_key(P.ar_base, (uint64_t)(__shfl_sync(0xffffffffu, ep_keep, (int)g) + 1u));
+                tA_keep = hasA ? d2d_draw_cue(key, genv, lane, P.cell_radius) : make_float2(1.f, 0.f);
+                pB_keep = hasB ? d2d_draw_due(key, genv, (C + 1u) >> 1, lane, P.cell_radius, P.d2d_radius) : make_float4(1.f, 0.f, 0.f, 0.f);
+                const uint4 ab = d2d_action_block(key, genv, lane, 0u);
+                aA = hasA ? __umulhi(d2d_action_word(ab, 0u, false), limA) : 0xffffffffu;
+                aB = hasB ? __umulhi(d2d_action_word(ab, 0u, true), limB) : 0xffffffffu;
+            }
+        }
         const float2 tA = tA_keep;
         const float4 pB = pB_keep;
         const uint32_t jA = iA + tN, jB = jA + C;                   // this env-step's link indices (outputs)
@@ -703,8 +734,9 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
         D2DLinkOut oA = oA32, oB = oB32;
         if (D2D_RESCUE_ENABLED && RESCUE_EARLY && __any_sync(0xffffffffu, needA || needB)) {
             const uint32_t keyA = liveA ? rbA : (D2D_INACTIVE_KEY | lane), keyB = liveB ? rbB : (D2D_INACTIVE_KEY | 32u | lane);
-            const uint32_t nr = (uint32_t)d2d_rescue_warp<PLE2, EXACT, SPEC, false, !FULL>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_, tA, pB, oA, oB);
-            st_resc += (ep_reset && t == 0u) ? 0u : nr;            // the reset step enters no statistic
+            const uint32_t nr = (uint32_t)d2d_rescue_warp<PLE2, EXACT, SPEC, false, !FULL, AR>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_, tA, pB,
+                                                                                                oA, oB, (AR && ar_rst));
+            st_resc += ((ep_reset && t == 0u) || (AR && ar_rst)) ? 0u : nr;   // the reset step enters no statistic
 #ifdef D2D_TIMELINE
             (tl_waited ? tl_post : tl_pre) += nr;
 #endif
@@ -713,15 +745,16 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
         // ---- per-warp statistics; flushed with the warp's LAST env, ahead of the wait and of that env's stores: the reductions
         // commute with every other launch's, and a warp (hence its block's slot) is not retired before its outstanding atomics
         // are acknowledged - issued at the very end they cost 0.3 us per launch of a one-wave batch (profiles/README.md) --------
-        if (!ep_reset || t != 0u) {                                 // the reset step (envs/d2d_env.py:50) earns no reward
+        if ((!ep_reset || t != 0u) && !(AR && ar_rst)) {                    // the reset step (envs/d2d_env.py:50) earns no reward
             if (P.reward_fn == 0) { st_reward += reward; st_reward2 = fmaf(reward, reward, st_reward2); }
             st_cap += cap_sum;
             st_pen += bad ? 1u : 0u;
+            if (AR) ++st_steps;
         }
         if (FLUSH_EARLY && P.stats && last_t && e + 1u == e_end && lane < (RESCUE_EARLY ? 6u : 5u)) {
             // one fire-and-forget fp64 reduction per statistic and warp, spread over the replicas
             const float vf = lane == 0 ? st_reward : lane == 1 ? st_cap : st_reward2;
-            const uint32_t vi = lane == 3 ? (e_end - e0) * (ep_reset ? T - 1u : T)  // env-steps this warp made
+            const uint32_t vi = lane == 3 ? (AR ? st_steps : (e_end - e0) * (ep_reset ? T - 1u : T))  // env-steps this warp made
                               : lane == 4 ? st_pen : st_resc;
             const double v = lane < 3u ? (double)vf : (double)vi;              // (two conversions instead of six)
 #ifndef D2D_EXPERIMENT_NOSTATS      // A/B only: what the statistics flush costs
@@ -740,7 +773,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
         // - another d2d_step of this handle - writes: they go out right away, and the wait moves in front of the only accesses that
         // do depend on the predecessor, the step counters and the per-env scalars of the warp's first group (see below).  At one wave
         // of envs every warp's stores used to queue up behind the grid-wide release.
-        const bool LATE = !MANY && (P.flags & D2D_PF_LATE_WAIT) != 0u;
+        const bool LATE = !MANY && !AR && (P.flags & D2D_PF_LATE_WAIT) != 0u;
         if (e == e0 && t == 0u && !LATE) {
             if (!MANY && P.tok_wait != 0ull) {
                 if (lane == 0u && !d2d_ticket_wait(P.tickets + (blockIdx.x * WPB + warp), P.tok_wait) && P.stats)
@@ -757,12 +790,12 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
 #ifdef D2D_EXPERIMENT_NOCOUNT     // A/B only: how much of the post-wait tail is the step-counter load
         ns_keep = 0;
 #else
-        if (!LATE && !ep_reset && g == 0u && t == 0u && (FULL || P.step_count)) ns_keep = e + lane < e_end ? (int)P.step_count[e + lane] : 0;   // consumed at the group's end
+        if (!AR && !LATE && !ep_reset && g == 0u && t == 0u && (FULL || P.step_count)) ns_keep = e + lane < e_end ? (int)P.step_count[e + lane] : 0;   // consumed at the group's end
 #endif
         // ---- outputs: compact observation table (envs/obs_fn.py:55-61), capacity, optional info.  Rows of absent
         // agents carry their positions and zeros (the reference has no row for them). ---------------------------------
         // (one divergent branch per slot: cheaper than predicating every store, and the two merge when C == D)
-        if (ep_reset && t == 0u) {
+        if ((ep_reset && t == 0u) || (AR && ar_rst)) {
             // the drawn positions become the bound state (after the wait: an earlier step kernel may still be reading it)
             float2 *pe = reinterpret_cast<float2 *>(P.pos_out) + (uint64_t)e * V;
             double2 *pe64 = P.pos64 ? reinterpret_cast<double2 *>(const_cast<double *>(P.pos64)) + (uint64_t)e * V : nullptr;
@@ -809,8 +842,9 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
         const auto rescue_late = [&]() {
             if (D2D_RESCUE_ENABLED && !RESCUE_EARLY && __any_sync(0xffffffffu, needA || needB)) {
                 const uint32_t keyA = liveA ? rbA : (D2D_INACTIVE_KEY | lane), keyB = liveB ? rbB : (D2D_INACTIVE_KEY | 32u | lane);
-                const uint32_t nr = (uint32_t)d2d_rescue_warp_late<PLE2, EXACT, SPEC, !FULL>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_, tA, pB);
-                st_resc += (ep_reset && t == 0u) ? 0u : nr;
+                const uint32_t nr = (uint32_t)d2d_rescue_warp_late<PLE2, EXACT, SPEC, !FULL, AR>(P, S, e, lane, jA, keyA, keyB, needA, needB, pA, pB_,
+                                                                                                  tA, pB, (AR && ar_rst));
+                st_resc += ((ep_reset && t == 0u) || (AR && ar_rst)) ? 0u : nr;
 #ifdef D2D_TIMELINE
                 (tl_waited ? tl_post : tl_pre) += nr;
 #endif
@@ -848,7 +882,8 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
                 if (last_t) ns_keep = ns;
             }
         } else {
-            rew_keep = lane == g ? reward : rew_keep;
+            rew_keep = lane == g ? ((AR && ar_rst) ? 0.f : reward) : rew_keep;
+            if (AR) rs_keep = lane == g ? (AR && ar_rst) : rs_keep;
         }
         if (last_t && (g == 31u || e + 1u == e_end)) {
             if (LATE) {
@@ -868,8 +903,9 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
             // envs/d2d_env.py:65,68 for the whole group: num_steps += 1; done = num_steps >= EPISODE_LENGTH
             if (lane <= g) {
                 const uint32_t eg = e - g + lane;
-                const int ns = MANY ? ns_keep : min(ns_keep + 1, 255);
+                const int ns = MANY ? ns_keep : (AR && rs_keep) ? 0 : min(ns_keep + 1, 255);
                 if (FULL || P.step_count) P.step_count[eg] = (uint8_t)ns;
+                if (AR && rs_keep) P.episode_index[eg] = ep_keep + 1u;
                 if (!MANY && (FULL || P.reward)) P.reward[eg] = rew_keep;
                 if (!MANY && (FULL || P.done)) P.done[eg] = ns >= P.episode_length ? 1 : 0;
             }
@@ -910,7 +946,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
     if (!FLUSH_EARLY) {
         if (P.stats && lane < 6u) {
             const float vf = lane == 0 ? st_reward : lane == 1 ? st_cap : st_reward2;
-            const uint32_t vi = lane == 3 ? (e_end - e0) * (ep_reset ? T - 1u : T) : lane == 4 ? st_pen : st_resc;
+            const uint32_t vi = lane == 3 ? (AR ? st_steps : (e_end - e0) * (ep_reset ? T - 1u : T)) : lane == 4 ? st_pen : st_resc;
             const double v = lane < 3u ? (double)vf : (double)vi;
             if (v != 0.0) atomicAdd(P.stats + ((blockIdx.x * WPB + warp) % D2D_STATS_REPLICAS) * 8 + lane, v);
         }

@@ -13,7 +13,7 @@
 namespace {
 constexpr int WPB = D2D_TU_WPB;
 
-// every instantiation d2d_step / d2d_step_many / d2d_episode may launch for this handle needs the dynamic shared-memory opt-in
+// every instantiation d2d_step (plain or auto-reset) / d2d_step_many / d2d_episode may launch for this handle needs the dynamic shared-memory opt-in
 template <bool PLE2, bool SPEC>
 int allow_all(size_t smem) {
     int rc = d2d_allow_smem(d2d_step_warp_kernel<PLE2, false, WPB, false, SPEC, 0>, smem);
@@ -25,6 +25,10 @@ int allow_all(size_t smem) {
     if (!rc) rc = d2d_allow_smem(d2d_step_warp_kernel<PLE2, false, WPB, false, SPEC, 2>, smem);
     if (!rc) rc = d2d_allow_smem(d2d_step_warp_kernel<PLE2, false, WPB, true, SPEC, 3>, smem);
     if (!rc) rc = d2d_allow_smem(d2d_step_warp_kernel<PLE2, false, WPB, true, SPEC, 4>, smem);
+    if (!rc) rc = d2d_allow_smem(d2d_step_warp_kernel<PLE2, false, WPB, false, SPEC, 5>, smem);
+    if (!rc) rc = d2d_allow_smem(d2d_step_warp_kernel<PLE2, false, WPB, true, SPEC, 5>, smem);
+    if (!rc) rc = d2d_allow_smem(d2d_step_warp_kernel<PLE2, true, WPB, false, SPEC, 5>, smem);
+    if (!rc) rc = d2d_allow_smem(d2d_step_warp_kernel<PLE2, true, WPB, true, SPEC, 5>, smem);
     return rc;
 }
 
@@ -35,6 +39,10 @@ cudaError_t launch(const D2DParams &P, int grid, size_t smem, const D2DLaunchSel
     if (sel.episode && sel.fast && sel.full) return sel.no_reset ? D2D_GO(false, true, 4) : D2D_GO(false, true, 3);
     if (sel.episode) return D2D_GO(false, false, 2);
     if (sel.many) return sel.exact ? D2D_GO(true, false, 1) : D2D_GO(false, false, 1);
+    if (sel.autoreset) {
+        if (sel.full) return sel.exact ? D2D_GO(true, true, 5) : D2D_GO(false, true, 5);
+        return sel.exact ? D2D_GO(true, false, 5) : D2D_GO(false, false, 5);
+    }
     if (sel.full) return sel.exact ? D2D_GO(true, true, 0) : D2D_GO(false, true, 0);
     return sel.exact ? D2D_GO(true, false, 0) : D2D_GO(false, false, 0);
 #undef D2D_GO

@@ -22,6 +22,18 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+_M64 = 0xFFFFFFFFFFFFFFFF
+
+
+def autoreset_key(base: int, n: int) -> int:
+    """Philox key of an env's n-th auto-reset under key base `base`: splitmix64(base + n * 0x9E3779B97F4A7C15), the library's
+    d2d_autoreset_key (gym_d2d_b200/csrc/d2d_common.cuh)."""
+    z = (int(base) + int(n) * 0x9E3779B97F4A7C15) & _M64
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & _M64
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & _M64
+    return z ^ (z >> 31)
+
+
 class StepBuffers:
     """One set of device output tensors of a step (the tensors a d2d_step_io_t points at)."""
 
@@ -64,10 +76,17 @@ class VecD2DEnv:
         reads the fp32 state; the shadow is read only by the kernels' rare fp64 recomputation path, so that
         results stay within 1e-4 relative of the reference evaluated on the caller's UNROUNDED float64
         positions (device-config files).  Not needed for positions drawn on the device by reset().
+    autoreset : next-step auto-reset (Gymnasium's AutoresetMode.NEXT_STEP) in step() and capture_steps().  An env whose previous
+        step returned done = 1 is reset by the next step instead of stepped: its actions in that call are ignored, and its row
+        of the results is the first observation of the new episode (new positions, the reset step's obs / capacity / info,
+        reward = 0, done = 0, step counter 0).  The reset draws positions and actions on the device under
+        autoreset_key(n), n = the env's entry of `episode_index` after the step.  Only configurations served by the warp
+        kernel (<= 32 CUEs, <= 32 DUE pairs, <= 64 RBs, no downlinks, no ShadowingPathLoss) support it; others raise here.
     """
 
     def __init__(self, num_envs: int, env_config: Optional[dict] = None, device: Any = 'cuda', seed: int = 0,
-                 global_env_offset: int = 0, info: bool = False, exact_positions: bool = False, downlink: bool = False) -> None:
+                 global_env_offset: int = 0, info: bool = False, exact_positions: bool = False, downlink: bool = False,
+                 autoreset: bool = False) -> None:
         env_config = env_config if env_config is not None else {}
         obs_enum = resolve_obs_fn(env_config.pop('obs_fn', LinearObsFunction))
         reward_enum, min_cap = resolve_reward_fn(env_config.pop('reward_fn', SystemCapacityRewardFunction))
@@ -116,6 +135,12 @@ class VecD2DEnv:
         self.positions_f64 = torch.zeros((E, V, 2), dtype=torch.float64, device=dev) if exact_positions else None
         if exact_positions:
             _lib.check(self._lib.d2d_bind_positions_f64(self._h, self.positions_f64.data_ptr()))
+        # auto-reset: episodes each env has begun since the last full reset() (int32, read as uint32 by the library)
+        self.autoreset = bool(autoreset)
+        self.episode_index = torch.zeros((E,), dtype=torch.int32, device=dev) if self.autoreset else None
+        self._ar_base = autoreset_key(self.seed, 0)      # until the first full reset() (see reset)
+        if self.autoreset:
+            self._bind_autoreset()
         # default output buffers, reused by every step (clone what you keep, or pass out=alloc_outputs())
         self._out = self.alloc_outputs()
         self.obs, self.capacity_mbps, self.reward, self.done = (self._out.obs, self._out.capacity_mbps,
@@ -131,6 +156,14 @@ class VecD2DEnv:
         _lib.check(self._lib.d2d_bind_state(self._h, self.positions.data_ptr(),
                                             self.step_count.data_ptr() if counted else None,
                                             self._stats.data_ptr() if counted else None))
+
+    def _bind_autoreset(self) -> None:
+        _lib.check(self._lib.d2d_bind_autoreset(self._h, self.episode_index.data_ptr(), self._ar_base))
+
+    def autoreset_key(self, n: int) -> int:
+        """Philox key of an env's n-th auto-reset since the last full reset() (the key d2d_reset / d2d_sample_actions would
+        take to draw the same positions and reset actions)."""
+        return autoreset_key(self._ar_base, n)
 
     def _stream(self) -> int:
         return torch.cuda.current_stream(self.device).cuda_stream
@@ -214,7 +247,9 @@ class VecD2DEnv:
         """Re-draw device positions on the GPU and zero the step counters (Simulator.reset, simulator.py:61-75;
         `num_steps = 0`, envs/d2d_env.py:46).  With mask=None this follows D2DEnv.reset (envs/d2d_env.py:45-52):
         one uncounted step with random actions produces the initial observation table, which is returned.
-        With a uint8/bool mask [E] only the flagged envs are re-drawn and nothing is returned."""
+        With a uint8/bool mask [E] only the flagged envs are re-drawn and nothing is returned.
+        With autoreset, a full reset also zeroes episode_index and makes this reset's key the base of the auto-reset keys;
+        reset(mask) leaves both alone (zeroing an env's index would make it repeat its own draws)."""
         if seed is not None:
             self.seed = int(seed)
             self._episode = 0
@@ -229,6 +264,12 @@ class VecD2DEnv:
         _lib.check(self._lib.d2d_reset(self._h, key, self.global_env_offset, _ptr(m), self._stream()))
         if mask is not None:
             return None
+        if self.autoreset:
+            self.episode_index.zero_()
+            # the base is this reset's key passed through splitmix64 once: reset keys advance by the same constant as the episode
+            # index inside autoreset_key, so with the raw key the next reset's stream would replay this one's shifted by an episode
+            self._ar_base = autoreset_key(key, 0)
+            self._bind_autoreset()
         actions = initial_actions if initial_actions is not None else self.sample_actions()
         self._bind(False)            # the reset step is not counted (simulator.step is called directly, :50)
         try:
@@ -238,14 +279,15 @@ class VecD2DEnv:
         return self.obs
 
     # ---- the hot path --------------------------------------------------------------------------
-    def _launch(self, actions: torch.Tensor, out: Optional[StepBuffers] = None, inputs_stable: bool = False) -> None:
+    def _launch(self, actions: torch.Tensor, out: Optional[StepBuffers] = None, inputs_stable: bool = False,
+                autoreset: bool = False) -> None:
         if actions.dtype != torch.int32 or not actions.is_cuda or not actions.is_contiguous():
             raise ValueError('actions must be a contiguous int32 CUDA tensor [num_envs][num_links]')
         if tuple(actions.shape) != (self.num_envs, self.num_links):
             raise ValueError(f'actions must have shape {(self.num_envs, self.num_links)}, got {tuple(actions.shape)}')
         io = (out if out is not None else self._out)._io
         io.actions = actions.data_ptr()
-        io.flags = _lib.STEP_INPUTS_STABLE if inputs_stable else 0
+        io.flags = (_lib.STEP_INPUTS_STABLE if inputs_stable else 0) | (_lib.STEP_AUTORESET if autoreset else 0)
         _lib.check(self._lib.d2d_step(self._h, C.byref(io), self._stream()))
 
     def step(self, actions: torch.Tensor, validate: bool = False, out: Optional[StepBuffers] = None,
@@ -257,13 +299,17 @@ class VecD2DEnv:
         read them while its predecessor is still running.  The default orders the step after everything earlier in the stream,
         which is what a loop whose policy writes the actions between steps needs.
 
+        With autoreset=True (constructor), envs whose previous step returned done are reset by this call instead: their actions
+        are ignored and their row is the first observation of the new episode (reward 0, done 0).  Such a step is always ordered
+        the default way, whatever inputs_stable says.
+
         actions: int32 [E][N]; < 0 marks an agent absent this step (Appendix B.8).  Returns the preallocated
         (obs [E][N][6], reward [E], done [E] uint8, info) tensors, overwritten by the next call.
         validate=True checks the action range on the device first (costs a host sync); out-of-range actions
         are otherwise the caller's responsibility (the reference accepts them silently, Appendix B.9)."""
         if validate and bool((actions >= self._nvec_dev.to(actions.dtype)).any()):
             raise ValueError('action out of range for its Discrete space')
-        self._launch(actions, out, inputs_stable)
+        self._launch(actions, out, inputs_stable, self.autoreset)
         o = out if out is not None else self._out
         info = {'capacity_mbps': o.capacity_mbps}
         if o.agent_reward is not None:
@@ -379,7 +425,9 @@ class VecD2DEnv:
         default buffers) into one CUDA graph: replay() then costs one launch for the whole sequence.
         inputs_stable: the action buffers are filled before every replay() and not rewritten during it (see step()); the
         first step of the graph is always ordered after whatever precedes the replay.  With ShadowingPathLoss the step-call
-        counter lives on the device, so every replay draws fresh shadowing values like the reference (path_loss.py:75-81)."""
+        counter lives on the device, so every replay draws fresh shadowing values like the reference (path_loss.py:75-81).
+        With autoreset the steps auto-reset finished envs like step(); episode_index lives on the device, so every replay draws
+        fresh positions (the key base is the one of the last full reset() before the capture)."""
         outs_seq = outs_seq if outs_seq is not None else [None] * len(actions_seq)
         graph = torch.cuda.CUDAGraph()
         side = torch.cuda.Stream(device=self.device)
@@ -387,7 +435,7 @@ class VecD2DEnv:
         with torch.cuda.stream(side):
             with torch.cuda.graph(graph, stream=side):
                 for a, o in zip(actions_seq, outs_seq):
-                    self._launch(a, o, inputs_stable)
+                    self._launch(a, o, inputs_stable, self.autoreset)
         torch.cuda.current_stream(self.device).wait_stream(side)
         return graph
 

@@ -43,6 +43,10 @@
  * anything enqueued ahead of the predecessor is complete.  Only the step counters and the per-env scalars (reward,
  * done) are written after the wait.  A caller that rotates two or more output sets gets this without asking; nothing
  * changes for one that reuses a single set.
+ * A step with D2D_STEP_AUTORESET is always ordered the default way, whatever D2D_STEP_INPUTS_STABLE says: it reads
+ * every input and the step counters after the wait, stores no output ahead of it and takes no per-warp ticket.  It
+ * also writes the positions of the envs it resets, so the step after it is ordered the default way too, as after
+ * d2d_episode.
  *
  * Index conventions (devices.py:20-25, simulator.py:34-48, envs/d2d_env.py:55-60):
  *   C = num_cues, D = num_due_pairs, N = C + D links, V = 1 + C + 2D devices.
@@ -144,6 +148,14 @@ typedef struct d2d_link {
                                        the reference fits: R n_pwr <= 32767; < 0 = agent absent) - half the upload per step; the library widens
                                        them on the device.  A host link shared by several GPUs gives the download what the upload leaves:
                                        profiles/README.md, "host link" */
+#define D2D_STEP_AUTORESET 4u       /* d2d_step only (warp-kernel configurations: <= 32 CUEs, <= 32 DUE pairs, <= 64 RBs, no downlinks, no
+                                       SHADOWING; D2D_ERR_UNSUPPORTED elsewhere and on every other step entry point): next-step auto-reset.
+                                       An env whose step counter is >= episode_length at entry (its previous step returned done = 1) is
+                                       reset instead of stepped, as d2d_reset + d2d_sample_actions(step 0) + one uncounted d2d_step would
+                                       do it, under the key of d2d_bind_autoreset; its actions in this call are ignored.  Its outputs
+                                       are that reset step's with reward = 0 and done = 0, its step counter becomes 0 and its episode
+                                       index goes up by 1; the reset step enters no statistic.  Needs d2d_bind_autoreset and a bound
+                                       step counter (D2D_ERR_STATE otherwise). */
 
 /* Buffers of one step.  All pointers are device pointers for d2d_step and host pointers for
  * d2d_step_host.  `actions` is required; any output may be NULL to skip it. */
@@ -197,6 +209,16 @@ D2D_API int d2d_state_bytes(const d2d_handle_t *h, size_t *positions_bytes, size
 /* Binds the device buffers that hold Device.position (device.py:48,82-83) for every env, D2DEnv.num_steps
  * (envs/d2d_env.py:43) and the statistics accumulators (stats may be NULL). */
 D2D_API int d2d_bind_state(d2d_handle_t *h, float *positions, uint8_t *step_count, double *stats);
+
+/* Binds what D2D_STEP_AUTORESET needs: episode_index uint32 [E] on the device (caller-owned; NULL unbinds) and the
+ * key base.  An env's n-th auto-reset (n = its episode index after the increment) draws its positions and actions under
+ * the Philox key splitmix64(base_key + n * 0x9E3779B97F4A7C15) (gym_d2d_b200/csrc/d2d_common.cuh: d2d_autoreset_key),
+ * with the global env in the counter: the draws depend on (base_key, global env, n) only, whatever the sharding or
+ * chunking, and a replayed CUDA graph draws fresh positions at every replay because episode_index lives on the device.
+ * Bases that advance by that same constant (keys seed + k * 0x9E3779B97F4A7C15) would make one base's stream the next one's
+ * shifted by an episode: mix them first (VecD2DEnv binds splitmix64 of its reset key).
+ * D2D_ERR_UNSUPPORTED on a configuration the warp kernel does not serve. */
+D2D_API int d2d_bind_autoreset(d2d_handle_t *h, uint32_t *episode_index, uint64_t base_key);
 
 /* Optional float64 shadow of the positions, float64 [E][V][2] (NULL unbinds).  When bound, d2d_set_positions /
  * d2d_reset also write it, and the step kernels read it in their rare fp64 recomputation path only: links whose
