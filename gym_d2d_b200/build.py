@@ -22,7 +22,7 @@ HEADER = PKG.parent / 'include' / 'd2d_b200.h'
 COMMON = ['d2d_internal.h', 'd2d_common.cuh']
 # (object name, source, extra defines, headers it includes besides COMMON)
 UNITS: List[Tuple[str, str, List[str], List[str]]] = [
-    ('abi', 'd2d_abi.cu', [], ['d2d_aux.cuh']),
+    ('abi', 'd2d_abi.cu', [], ['d2d_aux.cuh', 'd2d_launch_plan.h']),
     ('warp2', 'd2d_tu_warp.cu', ['-DD2D_TU_WPB=2'], ['d2d_step_warp.cuh']),
     ('warp4', 'd2d_tu_warp.cu', ['-DD2D_TU_WPB=4'], ['d2d_step_warp.cuh']),
     ('warp8', 'd2d_tu_warp.cu', ['-DD2D_TU_WPB=8'], ['d2d_step_warp.cuh']),

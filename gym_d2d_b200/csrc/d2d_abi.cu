@@ -11,6 +11,7 @@
 
 #include "d2d_internal.h"
 #include "d2d_aux.cuh"
+#include "d2d_launch_plan.h"
 
 static_assert(D2D_STATS_REPLICAS * 8 * sizeof(double) == 65536, "stats layout");
 
@@ -225,33 +226,34 @@ D2D_API int d2d_create(const d2d_config_t *cfg, const d2d_link_t *links, d2d_han
     h->use_warp = cfg->num_cues <= 32 && cfg->num_due_pairs <= 32 && cfg->num_rbs <= 64 && !general;
     if (const char *c = std::getenv("D2D_B200_CHUNK")) h->chunk_override = std::atoll(c);
     if (const char *c = std::getenv("D2D_B200_TICKET")) h->tickets_on = std::atoi(c) != 0;
-    if (const char *c = std::getenv("D2D_B200_TICKET_MIN")) h->ticket_min_quarters = std::max(1, std::atoi(c));
     if (const char *c = std::getenv("D2D_B200_LATE_WAIT")) h->late_wait_on = std::atoi(c) != 0;      // tests / A-B
     const char *pdl = std::getenv("D2D_B200_PDL");
     h->pdl = !(pdl && std::strcmp(pdl, "0") == 0);
+    const char *sp = std::getenv("D2D_B200_SPEC");
+    const bool spec_ok = !sp || std::atoi(sp) != 0;       // tests: D2D_B200_SPEC=0 forces the generic shapes
     int rc;
     if (h->use_warp) {
         // launch shape by batch size (d2d_step_warp.cuh): well under one wave of envs -> 2-warp blocks, everything else 4-warp blocks
         // (8-warp blocks were the large-batch shape until chains of steps stopped waiting for whole grids: with per-warp tickets
         // the 4-warp shape's 28 resident warps per SM win at every size - E = 131 072: 63.5 vs 65.9 us; D2D_B200_WPB=8 still selects it)
-        h->wpb = cfg->num_envs <= D2D_LATENCY_ENVS ? 2 : 4;
-        if (const char *w = std::getenv("D2D_B200_WPB")) { const int v = std::atoi(w); h->wpb = v == 8 ? 8 : v == 2 ? 2 : 4; }
-        h->spec = h->ple2 && h->uniform && cfg->path_loss_model != D2D_PL_COST_HATA && cfg->num_rbs == 25 && cfg->num_cues == 25 && cfg->num_due_pairs == 25 && cfg->n_pwr_cue == 24 &&
-                  cfg->n_pwr_due == 21;
-        if (const char *sp = std::getenv("D2D_B200_SPEC")) h->spec = h->spec && std::atoi(sp) != 0;   // tests: force the generic shape
-        // the fp64 pass reads 10^(p/10) from the constant bank of the translation unit that holds this shape's kernels
-        // (per device: set at every create)
-        cudaError_t et = h->wpb == 8 ? d2d_warp_tables_8(pwr_d) : h->wpb == 2 ? d2d_warp_tables_2(pwr_d) : d2d_warp_tables_4(pwr_d);
-        if (et != cudaSuccess) return bail(fail(D2D_ERR_CUDA, std::string("cudaMemcpyToSymbol(d2d_pwr_lin_c): ") + cudaGetErrorString(et)));
-        const size_t smem = h->wpb == 8 ? d2d_warp_smem_8(cfg->num_rbs) : h->wpb == 2 ? d2d_warp_smem_2(cfg->num_rbs) : d2d_warp_smem_4(cfg->num_rbs);
-        if (h->wpb == 4 && cfg->num_envs >= 65536 && !std::getenv("D2D_B200_WPB")) {      // the fused launches' own shape
-            et = d2d_warp_tables_8(pwr_d);
-            if (et != cudaSuccess) return bail(fail(D2D_ERR_CUDA, std::string("cudaMemcpyToSymbol(d2d_pwr_lin_c): ") + cudaGetErrorString(et)));
-            rc = d2d_warp_plan_8(h, d2d_warp_smem_8(cfg->num_rbs));
+        const char *w = std::getenv("D2D_B200_WPB");
+        h->warp = d2d_warp_shape(w ? std::atoi(w) : cfg->num_envs <= D2D_LATENCY_ENVS ? 2 : 4);
+        if (h->warp->wpb == 4 && cfg->num_envs >= 65536 && !w) h->many.warp = &d2d_warp_shape_8;     // the fused launches' own shape
+        h->spec = spec_ok && h->ple2 && h->uniform && cfg->path_loss_model != D2D_PL_COST_HATA && cfg->num_rbs == 25 && cfg->num_cues == 25 &&
+                  cfg->num_due_pairs == 25 && cfg->n_pwr_cue == 24 && cfg->n_pwr_due == 21;
+        // per shape this handle launches: the fp64 pass reads 10^(p/10) from the constant bank of the translation unit that holds
+        // the shape's kernels (per device: set at every create); then the geometry, in h->grid / block / smem / envs_per_block
+        auto setup = [&](const D2DWarpShape *ws) {
+            const cudaError_t et = ws->tables(pwr_d);
+            if (et != cudaSuccess) return fail(D2D_ERR_CUDA, std::string("cudaMemcpyToSymbol(d2d_pwr_lin_c): ") + cudaGetErrorString(et));
+            return ws->plan(h, ws->smem(cfg->num_rbs));
+        };
+        if (h->many.warp) {
+            rc = setup(h->many.warp);
             if (rc != D2D_OK) return bail(rc);
-            h->many.wpb = 8; h->many.grid = h->grid; h->many.smem = h->smem; h->many.envs_per_block = h->envs_per_block;
+            h->many.grid = h->grid; h->many.envs_per_block = h->envs_per_block;
         }
-        rc = h->wpb == 8 ? d2d_warp_plan_8(h, smem) : h->wpb == 2 ? d2d_warp_plan_2(h, smem) : d2d_warp_plan_4(h, smem);
+        rc = setup(h->warp);
     } else {
         // <= 1024 links: the binned one-barrier kernel (d2d_step_dense.cuh), LPT links per thread; when its double-buffered
         // bins do not fit (many RBs) the sorting block kernel; beyond 1024 links / other topologies: everything staged in shared memory
@@ -262,17 +264,15 @@ D2D_API int d2d_create(const d2d_config_t *cfg, const d2d_link_t *links, d2d_han
         // threads per block / links per thread: the shape with the fewest (warp, slot) bodies per env - every warp runs the
         // straight-line code of each of its slots whether or not all 32 lanes hold a link (N = 600: 10 warps x 2 slots,
         // all but one full, instead of 8 warps x 3 with the third slot three-quarters empty)
-        int bt = ((h->N + 319) / 320) * 10 < ((h->N + 255) / 256) * 8 && (h->N + 319) / 320 <= 3 ? 320 : 256;
-        if (dn && std::atoi(dn) >= 64) bt = std::atoi(dn);
+        const int bt = ((h->N + 319) / 320) * 10 < ((h->N + 255) / 256) * 8 && (h->N + 319) / 320 <= 3 ? 320 : 256;
         const bool dense = h->lpt > 0 && cfg->num_rbs <= 512 /* 9 bits of the packed link state */ &&
                            d2d_dense_smem(h->N, cfg->num_rbs, h->bin_cap, bt, h->V) <= 75 * 1024 /* three blocks per SM */ && !(dn && std::atoi(dn) == 0);
         if (dense) {
             h->dense_bt = bt;
             h->lpt = (h->N + bt - 1) / bt;
             // BASELINE config #3's shape has its own instantiation (d2d_step_dense.cuh: SPEC)
-            h->spec = h->ple2 && bt == 320 && h->N == 600 && cfg->num_cues == 100 && cfg->num_rbs == 100 && h->bin_cap == 16 && cfg->n_pwr_cue == 24 &&
-                      cfg->n_pwr_due == 21;
-            if (const char *sp = std::getenv("D2D_B200_SPEC")) h->spec = h->spec && std::atoi(sp) != 0;   // tests: force the generic shape
+            h->spec = spec_ok && h->ple2 && bt == 320 && h->N == 600 && cfg->num_cues == 100 && cfg->num_rbs == 100 && h->bin_cap == 16 &&
+                      cfg->n_pwr_cue == 24 && cfg->n_pwr_due == 21;
         }
         const size_t smem = dense ? d2d_dense_smem(h->N, cfg->num_rbs, h->bin_cap, bt, h->V) : d2d_block_smem(h->N, cfg->num_rbs, h->lpt);
         if (smem > 227 * 1024) return bail(fail(D2D_ERR_UNSUPPORTED, "d2d_create: too many links / RBs for one SM's shared memory"));
@@ -300,17 +300,15 @@ D2D_API int d2d_create(const d2d_config_t *cfg, const d2d_link_t *links, d2d_han
     // full grid; 10 steps: 4.7 / 5.3 / 5.5).  Large batches need every warp slot for their own latency hiding (E = 32 768: 17.1 us on
     // the full grid, 17.8 on three blocks per SM).  The latency shape (2-warp blocks): two blocks per SM - E = 1024 1.87 -> 1.76 us,
     // E = 2048 3.38 -> 2.32 us.  Sweeps: profiles/ab_r02_40.log .. ab_r02_46.log
-    if (h->use_warp && h->wpb == 2) h->grid_late = 2 * h->num_sms;
-    if (h->use_warp && h->wpb == 4) h->grid_late = cfg->num_envs <= 166 * (int64_t)h->num_sms ? 3 * h->num_sms : 0;
-    // (default-ordering steps keep the full grid: two envs per warp on half the blocks - D2D_B200_FRESH_GRID = ceil(E / 8) - speeds up
-    // back-to-back chains of them, E = 4096 10.6 -> 8.3 us, E = 6144 14.4 -> 9.7 us, but costs an isolated step behind a policy
-    // kernel 0.7 - 1 us, E = 2560 9.9 -> 10.9 us per pair: profiles/ab_r02_60.log)
-    if (const char *gf = std::getenv("D2D_B200_FRESH_GRID")) h->grid_fresh = std::max(0, std::atoi(gf));    // A/B
+    if (h->use_warp && h->warp->wpb == 2) h->grid_late = 2 * h->num_sms;
+    if (h->use_warp && h->warp->wpb == 4) h->grid_late = cfg->num_envs <= 166 * (int64_t)h->num_sms ? 3 * h->num_sms : 0;
+    // (default-ordering steps keep the full grid: half of it speeds up chains of them but costs an isolated step behind a policy
+    // kernel up to 1 us, profiles/README.md)
     if (const char *gl = std::getenv("D2D_B200_LATE_GRID")) h->grid_late = std::max(0, std::atoi(gl));      // A/B
     if (const char *gs = std::getenv("D2D_B200_GRID"))      // tests: few blocks, so every block steps many envs
         if (std::atoi(gs) > 0) { h->grid = std::min(h->grid, std::atoi(gs)); h->many.grid = std::min(h->many.grid, std::atoi(gs)); }
     if (h->use_warp) {      // one ticket word per warp slot of the step geometry
-        const size_t words = (size_t)h->grid * h->wpb;
+        const size_t words = (size_t)h->grid * h->warp->wpb;
         cudaError_t et = cudaMalloc(&h->dTickets, words * sizeof(uint64_t));
         if (et == cudaSuccess) et = cudaMemset(h->dTickets, 0, words * sizeof(uint64_t));
         if (et != cudaSuccess) return bail(fail(D2D_ERR_CUDA, std::string("ticket buffer: ") + cudaGetErrorString(et)));
@@ -342,7 +340,7 @@ D2D_API int d2d_destroy(d2d_handle_t *h) {
         for (void *p : s.stage) cudaFree(p);
         if (h->pipe_ready) { cudaEventDestroy(s.ev_in); cudaEventDestroy(s.ev_kernel); cudaEventDestroy(s.ev_out); }
     }
-    if (h->pipe_ready) { cudaStreamDestroy(h->s_in); cudaStreamDestroy(h->s_out); if (h->s_out2) cudaStreamDestroy(h->s_out2); }
+    if (h->pipe_ready) { cudaStreamDestroy(h->s_in); cudaStreamDestroy(h->s_out); }
     delete h;
     return D2D_OK;
 }
@@ -487,8 +485,6 @@ D2D_API int d2d_sample_actions(d2d_handle_t *h, int32_t *actions, uint64_t seed,
 
 namespace {
 
-enum { MODE_STEP = 0, MODE_MANY = 1, MODE_EPISODE = 2 };
-
 // per-agent rewards (SHANNON / CUE_SINR_SHANNON always; SYSTEM_CAPACITY when the caller asked for the broadcast): one more
 // small kernel over `total` env-steps of io; `with_stats`: the reward statistics of the per-agent functions; `autoreset`: rows
 // whose step counter is 0 after the step were reset by it (D2D_STEP_AUTORESET) and score nothing
@@ -512,105 +508,30 @@ int agent_reward_launch(d2d_handle *h, const d2d_step_io_t *io, int64_t total, b
     return D2D_OK;
 }
 
-// One launch (per chunk of envs) that makes T consecutive steps: MODE_STEP (T = 1) is d2d_step; MODE_MANY / MODE_EPISODE need
-// the warp kernel (T slices per env; the episode's slice 0 is the uncounted reset step).
-struct EpisodeArgs {
-    uint64_t ep_seed = 0, act_seed = 0;
-    uint32_t act_t0 = 0;         // step index of slice 0 in the action draws
-    bool draw_actions = false;
-    bool no_reset = false;       // d2d_rollout: continue from the bound state, every slice counted
-};
-
 int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *stream, const EpisodeArgs &ea = EpisodeArgs()) {
+    const D2DStepPlan pl = d2d_plan_step(h, io, mode, stream, ea);
     D2DParams P = make_params(h, io);
     P.T = T;
     P.t_stride = h->cfg.num_envs;
     P.ep_seed = ea.ep_seed; P.act_seed = ea.act_seed; P.act_t0 = ea.act_t0;
-    const bool draw_actions = ea.draw_actions;
+    P.flags = pl.flags | (ea.draw_actions ? D2D_PF_DRAW_ACTIONS : 0u) | (ea.no_reset ? D2D_PF_NO_RESET : 0u);
+    if (pl.tok_sign) { P.tickets = h->dTickets; P.tok_wait = pl.tok_wait; P.tok_sign = pl.tok_sign; }
     cudaStream_t st = (cudaStream_t)stream;
-    const bool many = mode != MODE_STEP;
-    // D2D_STEP_AUTORESET (d2d_step only): always the default ordering - wait at entry, no late wait, no tickets, the full grid
-    const bool autoreset = mode == MODE_STEP && (io->flags & D2D_STEP_AUTORESET) != 0u;
-    // "Ordering rule" of include/d2d_b200.h: inputs may be read ahead of griddepcontrol.wait only on the caller's promise AND when
-    // the kernel before this one (for this handle, in this stream) was a step kernel, which writes neither actions nor positions.
-    // An episode that draws its own actions reads no input at all.
-    // An episode that draws its own actions reads no input at all; a rollout reads the positions like a step does.
-    bool stable = h->pdl && h->last_stream == stream;
-    const bool reads_positions = mode != MODE_EPISODE || ea.no_reset;
-    if (!reads_positions && draw_actions) stable = h->pdl;
-    else if (!reads_positions) stable = stable && (io->flags & D2D_STEP_INPUTS_STABLE) && h->last_kind != D2D_LAST_OTHER;
-    else stable = stable && (io->flags & D2D_STEP_INPUTS_STABLE) && h->last_kind == D2D_LAST_STEP && !autoreset;
-    P.flags = (stable ? 0u : D2D_PF_INPUTS_FRESH) | (draw_actions ? D2D_PF_DRAW_ACTIONS : 0u) | (ea.no_reset ? D2D_PF_NO_RESET : 0u);
-    // Late wait (d2d_step_warp.cuh): a flagged single-launch d2d_step right behind another one of this handle, whose per-link output
-    // buffers alias none of the previous step's, stores them ahead of griddepcontrol.wait - nothing the predecessor does can
-    // collide with them, and whatever was enqueued before the predecessor is complete (a kernel that is not a step kernel never
-    // lets its successor start early).  The step counters and per-env scalars stay behind the wait.  Not when a post-pass kernel
-    // follows the step kernel.
-    // (measured, profiles/ab_r02_25 .. 28.log: a win at every batch size - E = 1 024: 2.55 -> 1.94 us, 4 096: 5.42 -> 4.94 us,
-    // 4 608: 7.76 -> 4.75 us, and level with or ahead of the per-warp tickets beyond one wave (E = 32 768: 17.8 -> 17.3 us) - except
-    // where two launches of 2-warp blocks fill the SM's warp slots exactly: E = 2 048 3.46 -> 4.22 us)
-    bool late = false;
-    {
-        const size_t EN = (size_t)h->cfg.num_envs * h->N;
-        const uintptr_t cur[6][2] = {{(uintptr_t)io->obs, EN * 24}, {(uintptr_t)io->obs_dyn, EN * 8}, {(uintptr_t)io->capacity_mbps, EN * 4},
-                                     {(uintptr_t)io->rate_bps, EN * 4}, {(uintptr_t)io->rb, EN * 2}, {(uintptr_t)io->tx_pwr_dBm, EN * 2}};
-        const bool plain = h->use_warp && mode == MODE_STEP && !autoreset && h->cfg.reward_fn == D2D_REWARD_SYSTEM_CAPACITY && !io->agent_reward && !h->dRngStep &&
-                           h->cfg.num_envs <= std::max<int64_t>(1, (int64_t)0x7fffffff / std::max(6 * h->N, 2 * h->V)) &&
-                           !(h->chunk_override > 0 && h->chunk_override < h->cfg.num_envs);
-        late = plain && stable && h->late_wait_on && h->prev_out_valid && h->last_kind == D2D_LAST_STEP && !(h->wpb == 2 && h->cfg.num_envs > 1792 && h->grid_late == 0);
-        for (int a = 0; late && a < 6; ++a)
-            for (int b = 0; b < 6; ++b)
-                if (cur[a][0] && h->prev_out[b][0] && cur[a][0] < h->prev_out[b][1] && h->prev_out[b][0] < cur[a][0] + cur[a][1]) late = false;
-        if (late) P.flags |= D2D_PF_LATE_WAIT;
-        h->prev_out_valid = plain;
-        for (int a = 0; a < 6; ++a) { h->prev_out[a][0] = cur[a][0]; h->prev_out[a][1] = cur[a][0] ? cur[a][0] + cur[a][1] : 0; }
-    }
-    // Per-warp tickets (d2d_common.cuh): a single-launch d2d_step publishes a token per warp; the next one - same stream, same
-    // geometry, inputs declared stable - waits per warp for that token instead of for the whole grid.
-    // (not when a post-pass kernel follows the step kernel: the next step's predecessor in the stream is then that kernel; and only
-    // for steps that write buffers their predecessor wrote - the late wait above serves the others)
-    const bool single_launch = !late && h->use_warp && mode == MODE_STEP && !autoreset && h->dTickets && h->pdl && h->tickets_on &&
-                               h->cfg.reward_fn == D2D_REWARD_SYSTEM_CAPACITY && !io->agent_reward && !h->dRngStep &&
-                               h->cfg.num_envs <= std::max<int64_t>(1, (int64_t)0x7fffffff / std::max(6 * h->N, 2 * h->V)) &&
-                               !(h->chunk_override > 0 && h->chunk_override < h->cfg.num_envs);
-    // (late: one chunk, never a fused launch; grid_fresh: an A/B knob, 0 by default - see d2d_create)
-    const int step_grid = late && h->grid_late > 0 ? std::min(h->grid, h->grid_late)
-                          : (!stable && mode == MODE_STEP && !autoreset && h->grid_fresh > 0) ? std::min(h->grid, h->grid_fresh) : h->grid;
-    const int grid1 = (int)std::min<int64_t>(step_grid, (h->cfg.num_envs + h->envs_per_block - 1) / h->envs_per_block);
-    // measured (profiles/README.md): the per-warp hand-off wins as soon as warps step more than one env per launch (E = 6 144,
-    // 1.5 envs per warp: 7.6 -> 5.3 us; E = 16 384: 12.4 -> 9.4 us; E = 131 072: 69.5 -> 65.9 us) and loses at exactly one
-    // (E = 4 096: 5.4 -> 6.8 us; E = 1 024: 2.7 -> 9.5 us), where the hardware's grid-wide wait stays - and where the launches do
-    // not publish tokens either (the release store holds a warp's block slot for an L2 round trip: 5.4 -> 10 us at E = 4 096)
-    const bool worth = 4 * h->cfg.num_envs >= (int64_t)h->ticket_min_quarters * grid1 * h->wpb;
-    if (single_launch && worth) {
-        const bool follow = stable && h->chain_seq > 0 && h->chain_seq < 0xffffu && h->chain_grid == grid1 && h->last_stream == stream;
-        if (!follow) { ++h->chain_id; h->chain_seq = 0; h->chain_grid = grid1; }
-        P.tickets = h->dTickets;
-        P.tok_wait = follow ? ((h->chain_id << 16) | h->chain_seq) : 0ull;
-        P.tok_sign = (h->chain_id << 16) | (h->chain_seq + 1u);
-        ++h->chain_seq;
-    } else {
-        h->chain_seq = 0;
-    }
-    // the kernels index with 32 bits: batches beyond 2^31 / (T max(6N, 2V)) envs (> 7 million default envs) go in chunks
-    int64_t chunk = std::max<int64_t>(1, (int64_t)0x7fffffff / std::max(6 * h->N, 2 * h->V));
-    if (many) chunk = h->cfg.num_envs;        // the callers checked that T slices fit 32-bit indices
-    if (h->chunk_override > 0 && !many) chunk = std::min(chunk, h->chunk_override);
-    for (int64_t e0 = 0; e0 < h->cfg.num_envs; e0 += chunk) {
-        const int64_t n = std::min<int64_t>(chunk, h->cfg.num_envs - e0);
+    for (int64_t e0 = 0; e0 < h->cfg.num_envs; e0 += pl.chunk) {
+        const int64_t n = std::min<int64_t>(pl.chunk, h->cfg.num_envs - e0);
         if (e0 > 0) {
-            const int64_t dl = chunk * h->N;
-            P.first_global_env += (uint64_t)chunk;
+            const int64_t dl = pl.chunk * h->N;
+            P.first_global_env += (uint64_t)pl.chunk;
             if (P.actions) P.actions += dl;
-            P.pos += chunk * h->V * 2; P.pos_out += chunk * h->V * 2;
-            if (P.pos64) P.pos64 += chunk * h->V * 2;
-            if (P.step_count) P.step_count += chunk;
-            if (P.episode_index) P.episode_index += chunk;
+            P.pos += pl.chunk * h->V * 2; P.pos_out += pl.chunk * h->V * 2;
+            if (P.pos64) P.pos64 += pl.chunk * h->V * 2;
+            if (P.step_count) P.step_count += pl.chunk;
+            if (P.episode_index) P.episode_index += pl.chunk;
             if (P.obs) P.obs += dl * 6;
             if (P.obs_dyn) P.obs_dyn += dl;
             if (P.cap) P.cap += dl;
-            if (P.reward) P.reward += chunk;
-            if (P.done) P.done += chunk;
+            if (P.reward) P.reward += pl.chunk;
+            if (P.done) P.done += pl.chunk;
             if (P.rate) P.rate += dl;
             if (P.rb_out) P.rb_out += dl;
             if (P.pwr_out) P.pwr_out += dl;
@@ -621,23 +542,22 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
 #ifdef D2D_TIMELINE
         P.tl_slot = (int32_t)(h->launches % D2D_TL_SLOTS);
 #endif
-        const bool alt = many && h->many.wpb != 0;               // fused multi-step launches of large batches: their own shape
-        const int wpb = alt ? h->many.wpb : h->wpb, epb = alt ? h->many.envs_per_block : h->envs_per_block;
-        const int grid = (int)std::min<int64_t>(alt ? h->many.grid : step_grid, (n + epb - 1) / epb);
-        if (h->use_warp) { const int64_t warps = (int64_t)grid * wpb; P.envs_per_warp = (uint32_t)(n / warps); P.envs_extra = (uint32_t)(n % warps); }
+        const bool alt = mode != MODE_STEP && h->many.warp;      // fused multi-step launches of large batches: their own shape
+        const D2DWarpShape *warp = alt ? h->many.warp : h->warp;
+        const int epb = alt ? h->many.envs_per_block : h->envs_per_block;
+        const int grid = (int)std::min<int64_t>(alt ? h->many.grid : pl.grid, (n + epb - 1) / epb);
+        if (h->use_warp) { const int64_t warps = (int64_t)grid * warp->wpb; P.envs_per_warp = (uint32_t)(n / warps); P.envs_extra = (uint32_t)(n % warps); }
         D2DLaunchSel sel;
         sel.many = mode == MODE_MANY; sel.episode = mode == MODE_EPISODE;
         sel.no_reset = ea.no_reset;
-        sel.autoreset = autoreset;
-        sel.fast = mode == MODE_EPISODE && draw_actions && !io->actions_out;
+        sel.autoreset = pl.autoreset;
+        sel.fast = mode == MODE_EPISODE && ea.draw_actions && !io->actions_out;
         sel.exact = h->pos64 != nullptr;
-        sel.smem = alt ? h->many.smem : h->smem;
         // FULL: exactly the core outputs were passed, so the kernel tests no output pointer on its hot path
         sel.full = io->obs && io->capacity_mbps && io->reward && io->done && !io->rate_bps && !io->rb && !io->tx_pwr_dBm && !io->obs_dyn &&
                    h->step_count && h->cfg.reward_fn == D2D_REWARD_SYSTEM_CAPACITY;
         cudaError_t err;
-        if (h->use_warp) err = wpb == 8 ? d2d_warp_launch_8(h, P, grid, sel, st, h->pdl) : wpb == 2 ? d2d_warp_launch_2(h, P, grid, sel, st, h->pdl)
-                                                                                                       : d2d_warp_launch_4(h, P, grid, sel, st, h->pdl);
+        if (h->use_warp) err = warp->launch(h, P, grid, sel, st, h->pdl);
         else if (h->dense_bt) err = d2d_dense_launch(h, P, grid, sel, st, h->pdl);
         else err = d2d_block_launch(h, P, grid, st, h->pdl);
         if (err != cudaSuccess) return fail(D2D_ERR_CUDA, std::string("step kernel launch: ") + cudaGetErrorString(err));
@@ -645,14 +565,13 @@ int step_launch(d2d_handle *h, const d2d_step_io_t *io, int T, int mode, void *s
     }
     D2D_CUDA(cudaGetLastError());
     h->last_stream = stream;
-    // (an auto-reset step wrote positions: the next step reads them after its wait, as after an episode)
-    h->last_kind = (mode == MODE_EPISODE && !ea.no_reset) || autoreset ? D2D_LAST_EPISODE : D2D_LAST_STEP;
+    h->last_kind = pl.last_kind;
     if (h->dRngStep) {      // ShadowingPathLoss: the next call draws fresh values, also when this one is replayed from a CUDA graph
         d2d_advance_counter_kernel<<<1, 1, 0, st>>>(h->dRngStep, (uint64_t)T);
         D2D_CUDA(cudaGetLastError());
     }
     if (mode != MODE_EPISODE && (h->cfg.reward_fn != D2D_REWARD_SYSTEM_CAPACITY || io->agent_reward))
-        return agent_reward_launch(h, io, (int64_t)T * h->cfg.num_envs, true, st, autoreset);
+        return agent_reward_launch(h, io, (int64_t)T * h->cfg.num_envs, true, st, pl.autoreset);
     return D2D_OK;
 }
 
@@ -669,6 +588,19 @@ int check_step_args(const d2d_handle_t *h, const d2d_step_io_t *io, const char *
         return fail(D2D_ERR_INVALID_ARG, std::string(who) + ": D2D_STEP_ACTIONS_I16 applies to d2d_step_host / d2d_step_host_async only");
     if (io->obs && ((uintptr_t)io->obs % 8)) return fail(D2D_ERR_INVALID_ARG, std::string(who) + ": obs must be 8-byte aligned");
     if (io->obs_dyn && ((uintptr_t)io->obs_dyn % 8)) return fail(D2D_ERR_INVALID_ARG, std::string(who) + ": obs_dyn must be 8-byte aligned");
+    return D2D_OK;
+}
+
+// d2d_episode / d2d_rollout: the per-agent reward pass and the composed path read drawn actions back; when the caller does not
+// record them, they go to handle-owned scratch of `slices` x E x N actions
+int reserve_act_scratch(d2d_handle *h, int64_t slices, cudaStream_t st) {
+    const size_t need = (size_t)slices * h->cfg.num_envs * h->N;
+    if (h->act_scratch_elems >= need) return D2D_OK;
+    D2D_CUDA(cudaStreamSynchronize(st));
+    cudaFree(h->act_scratch);
+    h->act_scratch = nullptr; h->act_scratch_elems = 0;
+    D2D_CUDA(cudaMalloc(&h->act_scratch, need * sizeof(int32_t)));
+    h->act_scratch_elems = need;
     return D2D_OK;
 }
 
@@ -702,11 +634,10 @@ D2D_API int d2d_step_many(d2d_handle_t *h, const d2d_step_io_t *io, int32_t num_
     if (rc) return rc;
     if (num_steps < 1) return fail(D2D_ERR_INVALID_ARG, "d2d_step_many: num_steps must be >= 1");
     D2D_GUARD(h);
-    const int64_t E = h->cfg.num_envs, per_env = std::max(6 * h->N, 2 * h->V);
+    const int64_t E = h->cfg.num_envs;
     // fused launches of as many steps as 32-bit indices allow (all of them unless T E N is astronomically large);
     // configurations served by the block kernel take one launch per step
-    int64_t fuse = h->use_warp ? std::min<int64_t>(num_steps, (int64_t)0x7fffffff / (E * per_env)) : 1;
-    if (fuse < 1) fuse = 1;
+    const int64_t fuse = h->use_warp ? std::clamp<int64_t>(d2d_max_launch_envs(h) / E, 1, num_steps) : 1;
     d2d_step_io_t cur = *io;
     for (int64_t t0 = 0; t0 < num_steps; t0 += fuse) {
         const int T = (int)std::min<int64_t>(fuse, num_steps - t0);
@@ -726,21 +657,14 @@ D2D_API int d2d_episode(d2d_handle_t *h, const d2d_step_io_t *io, int32_t num_st
     if (!h->step_count) return fail(D2D_ERR_STATE, "d2d_episode: a step-counter buffer must be bound");
     D2D_GUARD(h);
     cudaStream_t st = (cudaStream_t)stream;
-    const int64_t E = h->cfg.num_envs, per_env = std::max(6 * h->N, 2 * h->V);
+    const int64_t E = h->cfg.num_envs;
     const int T1 = num_steps + 1;
     const bool agent_pass = h->cfg.reward_fn != D2D_REWARD_SYSTEM_CAPACITY || io->agent_reward;
     d2d_step_io_t cur = *io;
-    const bool fused = h->use_warp && (int64_t)T1 * E * per_env <= (int64_t)0x7fffffff;
-    // the per-agent reward pass and the composed path read the actions back: record drawn ones in handle-owned scratch
+    const bool fused = h->use_warp && (int64_t)T1 * E <= d2d_max_launch_envs(h);
     if (draw && !cur.actions_out && (agent_pass || !fused)) {
-        const size_t need = (size_t)(fused ? T1 : 1) * E * h->N;
-        if (h->act_scratch_elems < need) {
-            D2D_CUDA(cudaStreamSynchronize(st));
-            cudaFree(h->act_scratch);
-            h->act_scratch = nullptr; h->act_scratch_elems = 0;
-            D2D_CUDA(cudaMalloc(&h->act_scratch, need * sizeof(int32_t)));
-            h->act_scratch_elems = need;
-        }
+        rc = reserve_act_scratch(h, fused ? T1 : 1, st);
+        if (rc) return rc;
     }
     if (fused) {
         if (draw && !cur.actions_out && agent_pass) cur.actions_out = h->act_scratch;
@@ -789,21 +713,15 @@ D2D_API int d2d_rollout(d2d_handle_t *h, const d2d_step_io_t *io, int32_t num_st
     if (num_steps < 1) return fail(D2D_ERR_INVALID_ARG, "d2d_rollout: num_steps must be >= 1");
     D2D_GUARD(h);
     cudaStream_t st = (cudaStream_t)stream;
-    const int64_t E = h->cfg.num_envs, per_env = std::max(6 * h->N, 2 * h->V);
+    const int64_t E = h->cfg.num_envs;
     const bool agent_pass = h->cfg.reward_fn != D2D_REWARD_SYSTEM_CAPACITY || io->agent_reward;
     d2d_step_io_t cur = *io;
     cur.actions = nullptr;
     // (with an fp64 position shadow bound the steps must run the shadow-aware instantiation: composed path)
-    const bool fused = h->use_warp && !h->pos64 && (int64_t)num_steps * E * per_env <= (int64_t)0x7fffffff;
+    const bool fused = h->use_warp && !h->pos64 && (int64_t)num_steps * E <= d2d_max_launch_envs(h);
     if (!cur.actions_out && (agent_pass || !fused)) {
-        const size_t need = (size_t)(fused ? num_steps : 1) * E * h->N;
-        if (h->act_scratch_elems < need) {
-            D2D_CUDA(cudaStreamSynchronize(st));
-            cudaFree(h->act_scratch);
-            h->act_scratch = nullptr; h->act_scratch_elems = 0;
-            D2D_CUDA(cudaMalloc(&h->act_scratch, need * sizeof(int32_t)));
-            h->act_scratch_elems = need;
-        }
+        rc = reserve_act_scratch(h, fused ? num_steps : 1, st);
+        if (rc) return rc;
     }
     if (fused) {
         if (!cur.actions_out && agent_pass) cur.actions_out = h->act_scratch;
@@ -836,7 +754,6 @@ int host_pipeline_init(d2d_handle *h) {
     if (h->pipe_ready) return D2D_OK;
     D2D_CUDA(cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking));
     D2D_CUDA(cudaStreamCreateWithFlags(&h->s_out, cudaStreamNonBlocking));
-    if (const char *c = std::getenv("D2D_B200_OUT_STREAMS")) if (std::atoi(c) == 2) D2D_CUDA(cudaStreamCreateWithFlags(&h->s_out2, cudaStreamNonBlocking));
     for (auto &s : h->slot) {
         D2D_CUDA(cudaEventCreateWithFlags(&s.ev_in, cudaEventDisableTiming));
         D2D_CUDA(cudaEventCreateWithFlags(&s.ev_kernel, cudaEventDisableTiming));
@@ -847,7 +764,6 @@ int host_pipeline_init(d2d_handle *h) {
 }
 
 // the buffers of a d2d_step_io_t in a fixed order: actions, then the outputs
-struct IoField { void *d2d_step_io_t::*dummy; };
 void io_pointers(const d2d_step_io_t *io, void *out[D2D_NUM_IO_BUFFERS]) {
     out[0] = (void *)io->actions; out[1] = io->obs; out[2] = io->obs_dyn; out[3] = io->capacity_mbps; out[4] = io->reward;
     out[5] = io->done; out[6] = io->rate_bps; out[7] = io->rb; out[8] = io->tx_pwr_dBm; out[9] = io->agent_reward;
@@ -955,17 +871,16 @@ D2D_API int d2d_step_host_async(d2d_handle_t *h, const d2d_step_io_t *hio, int s
     if (rc) return rc;
     D2D_CUDA(cudaEventRecord(s.ev_kernel, st));
     // copy-out
-    cudaStream_t so = (h->s_out2 && (slot & 1)) ? h->s_out2 : h->s_out;
-    D2D_CUDA(cudaStreamWaitEvent(so, s.ev_kernel, 0));
+    D2D_CUDA(cudaStreamWaitEvent(h->s_out, s.ev_kernel, 0));
     if (packed) {
-        D2D_CUDA(cudaMemcpyAsync((char *)s.host + s.out_offset, (char *)s.dev + s.out_offset, s.out_bytes, cudaMemcpyDeviceToHost, so));
+        D2D_CUDA(cudaMemcpyAsync((char *)s.host + s.out_offset, (char *)s.dev + s.out_offset, s.out_bytes, cudaMemcpyDeviceToHost, h->s_out));
     } else {
         void *dp[D2D_NUM_IO_BUFFERS];
         io_pointers(&dio, dp);
         for (int i = 1; i < D2D_NUM_IO_BUFFERS; ++i)
-            if (host[i]) D2D_CUDA(cudaMemcpyAsync(host[i], dp[i], bytes[i], cudaMemcpyDeviceToHost, so));
+            if (host[i]) D2D_CUDA(cudaMemcpyAsync(host[i], dp[i], bytes[i], cudaMemcpyDeviceToHost, h->s_out));
     }
-    D2D_CUDA(cudaEventRecord(s.ev_out, so));
+    D2D_CUDA(cudaEventRecord(s.ev_out, h->s_out));
     s.used = true;
     return D2D_OK;
 }
@@ -1008,7 +923,7 @@ D2D_API int d2d_stats_reset(d2d_handle_t *h, void *stream) {
 // instrumented build only (profiles/timeline.py): copies the stamp table to the host
 D2D_API int d2d_debug_timeline(void *host_out, size_t bytes, int wpb) {
     D2D_CUDA(cudaDeviceSynchronize());
-    D2D_CUDA(wpb == 8 ? d2d_warp_timeline_8(host_out, bytes) : wpb == 2 ? d2d_warp_timeline_2(host_out, bytes) : d2d_warp_timeline_4(host_out, bytes));
+    D2D_CUDA(d2d_warp_shape(wpb)->timeline(host_out, bytes));
     return D2D_OK;
 }
 #endif

@@ -48,7 +48,7 @@ struct d2d_handle {
     D2DLinkA u_cue{}, u_due{};
     D2DLinkD ud_cue{}, ud_due{};
     float us_cue[2] = {0, 0}, us_due[2] = {0, 0};
-    int wpb = 4;               // warps per block of the warp kernel
+    const struct D2DWarpShape *warp = nullptr;   // warp kernel: the shape of the step geometry (nullptr: another kernel family)
     int dense_bt = 0;          // dense kernel (d2d_step_dense.cuh): threads per block, 0 = not used
     int bin_cap = 0;           // dense kernel: record slots per RB bin
     int lpt = 0;               // block / dense kernel: links per thread held in registers (0 = the generic shared-memory kernel)
@@ -57,8 +57,8 @@ struct d2d_handle {
     int grid = 0, block = 0, smem = 0, envs_per_block = 0;
     // second geometry of the warp kernel for the fused multi-step launches (d2d_step_many / d2d_episode / d2d_rollout) of large
     // batches: their warps run for hundreds of microseconds and never hand over per step, and there 8-warp blocks measured
-    // better than the 4-warp shape the single steps use (episode at E = 131 072: 785 vs 830 us); wpb = 0: same geometry as the steps
-    struct { int wpb = 0, grid = 0, smem = 0, envs_per_block = 0; } many;
+    // better than the 4-warp shape the single steps use (episode at E = 131 072: 785 vs 830 us); warp = nullptr: same geometry as the steps
+    struct { const D2DWarpShape *warp = nullptr; int grid = 0, envs_per_block = 0; } many;
     double K_dB = 0.0, ple = 2.0;
     D2DLinkA *dA = nullptr;
     D2DLinkB *dB = nullptr;
@@ -77,22 +77,21 @@ struct d2d_handle {
     uint64_t ar_base = 0;
     // host-buffer steps (d2d_step_host*): the pipeline slots
     d2d_host_slot slot[D2D_HOST_SLOTS];
-    cudaStream_t s_in = nullptr, s_out = nullptr, s_out2 = nullptr;      // s_out2: odd slots' copy-out (D2D_B200_OUT_STREAMS=2, A/B)
+    cudaStream_t s_in = nullptr, s_out = nullptr;
     bool pipe_ready = false;
     double *stage_pos = nullptr;
     int64_t stage_pos_envs = 0;
     int64_t launches = 0;
-    // programmatic dependent launch bookkeeping (include/d2d_b200.h, "Ordering rule"): the stream of the last kernel this
-    // handle enqueued and whether that kernel was one of its own step kernels (anything else - reset, set_positions -
-    // wrote state a step kernel reads ahead of griddepcontrol.wait)
+    // programmatic dependent launch bookkeeping (include/d2d_b200.h, "Ordering rule"; kept by d2d_plan_step, d2d_launch_plan.h):
+    // the stream of the last kernel this handle enqueued and whether that kernel was one of its own step kernels (anything
+    // else - reset, set_positions - wrote state a step kernel reads ahead of griddepcontrol.wait)
     void *last_stream = nullptr;
     int last_kind = 0;             // D2D_LAST_*
-    // the per-link output buffers of the last single-launch d2d_step ([begin, end) byte ranges; obs, obs_dyn, capacity, rate, rb,
+    // the per-link output buffers of the last single-kernel plain step ([begin, end) byte ranges; obs, obs_dyn, capacity, rate, rb,
     // Tx power): a d2d_step right behind it that touches none of them stores its own ahead of griddepcontrol.wait (D2D_PF_LATE_WAIT)
     uintptr_t prev_out[6][2] = {};
     bool prev_out_valid = false;
     bool late_wait_on = true;      // D2D_B200_LATE_WAIT=0 switches the late wait off (tests, A/B)
-    int grid_fresh = 0;            // warp kernel: blocks of a default-ordering step (0 = the full grid; D2D_B200_FRESH_GRID, A/B only)
     int grid_late = 0;             // warp kernel: blocks of a late-wait step (0 = the full grid).  Under the late wait consecutive steps overlap
                                    // for as long as the SMs have room for both: a launch that leaves the larger part of the block slots free
                                    // lets its successor's blocks start while its own are still running (d2d_abi.cu, DESIGN.md 4.7)
@@ -103,8 +102,6 @@ struct d2d_handle {
     uint32_t chain_seq = 0;        // tokens published so far in this chain (0: the previous launch was not a signing step)
     int chain_grid = 0;            // grid of the chain's launches
     bool tickets_on = true;        // D2D_B200_TICKET=0 disables (A/B, tests)
-    int ticket_min_quarters = 5;   // D2D_B200_TICKET_MIN: tickets from this many QUARTER envs per warp (5 = 1.25 envs): with one env per
-                                   // warp the hardware's grid-wide wait is cheaper than the release / acquire hand-off (two L2 round trips)
     // d2d_episode: handle-owned scratch for drawn actions when the caller does not ask for them but a later pass needs them
     int32_t *act_scratch = nullptr;
     size_t act_scratch_elems = 0;
@@ -183,22 +180,22 @@ struct D2DLaunchSel {
     bool fast = false;       // ... with drawn actions, no action record and no fp64 shadow: the compiled-in variants
     bool no_reset = false;   // ... d2d_rollout
     bool autoreset = false;  // d2d_step with D2D_STEP_AUTORESET (warp kernel only)
-    int smem = 0;            // dynamic shared memory of the geometry this launch uses
 };
 
-// warp kernel (d2d_step_warp.cuh), one TU per warps-per-block shape
+// warp kernel (d2d_step_warp.cuh): one TU, and one table of its entry points, per warps-per-block shape (d2d_tu_warp.cu)
 #ifndef D2D_LATENCY_ENVS
 #define D2D_LATENCY_ENVS 2048      // batches up to this size take the 2-warp latency shape (d2d_step_warp.cuh)
 #endif
-#define D2D_DECLARE_WARP_TU(WPB)                                                                                        \
-    size_t d2d_warp_smem_##WPB(int R);                                                                                  \
-    int d2d_warp_plan_##WPB(d2d_handle *h, size_t smem);                                                                \
-    cudaError_t d2d_warp_launch_##WPB(const d2d_handle *h, const D2DParams &P, int grid, const D2DLaunchSel &sel, cudaStream_t st, bool pdl); \
-    cudaError_t d2d_warp_tables_##WPB(const double *pwr_lin_d);                                                         \
-    cudaError_t d2d_warp_timeline_##WPB(void *host_out, size_t bytes);      /* instrumented builds only (-DD2D_TIMELINE) */
-D2D_DECLARE_WARP_TU(2)
-D2D_DECLARE_WARP_TU(4)
-D2D_DECLARE_WARP_TU(8)
+struct D2DWarpShape {
+    int wpb;                                                   // warps per block
+    size_t (*smem)(int R);                                     // dynamic shared memory per block for R RBs
+    int (*plan)(d2d_handle *h, size_t smem);                   // shared-memory opt-in of every instantiation, h->grid / block / smem / envs_per_block
+    cudaError_t (*launch)(const d2d_handle *h, const D2DParams &P, int grid, const D2DLaunchSel &sel, cudaStream_t st, bool pdl);
+    cudaError_t (*tables)(const double *pwr_lin_d);            // 10^(p/10) into the TU's constant bank (per device: at every create)
+    cudaError_t (*timeline)(void *host_out, size_t bytes);     // the TU's stamp table (-DD2D_TIMELINE builds; nullptr otherwise)
+};
+extern const D2DWarpShape d2d_warp_shape_2, d2d_warp_shape_4, d2d_warp_shape_8;
+inline const D2DWarpShape *d2d_warp_shape(int wpb) { return wpb == 8 ? &d2d_warp_shape_8 : wpb == 2 ? &d2d_warp_shape_2 : &d2d_warp_shape_4; }
 
 // dense kernel (d2d_step_dense.cuh)
 size_t d2d_dense_smem(int N, int R, int bin_cap, int bt, int V);

@@ -757,9 +757,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
             const uint32_t vi = lane == 3 ? (AR ? st_steps : (e_end - e0) * (ep_reset ? T - 1u : T))  // env-steps this warp made
                               : lane == 4 ? st_pen : st_resc;
             const double v = lane < 3u ? (double)vf : (double)vi;              // (two conversions instead of six)
-#ifndef D2D_EXPERIMENT_NOSTATS      // A/B only: what the statistics flush costs
             if (v != 0.0) atomicAdd(P.stats + ((blockIdx.x * WPB + warp) % D2D_STATS_REPLICAS) * 8 + lane, v);
-#endif
         }
 
         // griddepcontrol.wait: everything above read only inputs (no step kernel writes actions or positions); from here on every
@@ -787,11 +785,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
         if (e == e0 && t == 0u) tl_c2 = d2d_tl_clock();
         if (e == e0 && t == 0u && !LATE) tl_waited = true;
 #endif
-#ifdef D2D_EXPERIMENT_NOCOUNT     // A/B only: how much of the post-wait tail is the step-counter load
-        ns_keep = 0;
-#else
         if (!AR && !LATE && !ep_reset && g == 0u && t == 0u && (FULL || P.step_count)) ns_keep = e + lane < e_end ? (int)P.step_count[e + lane] : 0;   // consumed at the group's end
-#endif
         // ---- outputs: compact observation table (envs/obs_fn.py:55-61), capacity, optional info.  Rows of absent
         // agents carry their positions and zeros (the reference has no row for them). ---------------------------------
         // (one divergent branch per slot: cheaper than predicating every store, and the two merge when C == D)
@@ -894,11 +888,7 @@ d2d_step_warp_kernel(const __grid_constant__ D2DParams P) {
 #ifdef D2D_TIMELINE
                 if (e - g == e0) { tl_c2 = d2d_tl_clock(); tl_waited = true; }
 #endif
-#ifdef D2D_EXPERIMENT_NOCOUNT
-                ns_keep = 0;
-#else
                 ns_keep = ((FULL || P.step_count) && lane <= g) ? (int)P.step_count[e - g + lane] : 0;
-#endif
             }
             // envs/d2d_env.py:65,68 for the whole group: num_steps += 1; done = num_steps >= EPISODE_LENGTH
             if (lane <= g) {

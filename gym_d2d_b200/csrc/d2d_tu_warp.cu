@@ -1,6 +1,6 @@
 // d2d_tu_warp.cu - the instantiations of d2d_step_warp_kernel for ONE warps-per-block shape (-DD2D_TU_WPB=2 | 4 | 8; the
-// library links three copies of this file, compiled in parallel).  Exports d2d_warp_plan_<WPB>, d2d_warp_launch_<WPB> and
-// d2d_warp_tables_<WPB> (d2d_internal.h).
+// library links three copies of this file, compiled in parallel).  Exports their entry points as the table
+// d2d_warp_shape_<WPB> (d2d_internal.h).
 #include "d2d_internal.h"
 #include "d2d_step_warp.cuh"
 
@@ -32,9 +32,11 @@ int allow_all(size_t smem) {
     return rc;
 }
 
+size_t shape_smem(int R) { return d2d_warp_smem_bytes(R, WPB); }
+
 template <bool PLE2, bool SPEC>
-cudaError_t launch(const D2DParams &P, int grid, size_t smem, const D2DLaunchSel &sel, cudaStream_t st, bool pdl) {
-#define D2D_GO(EXACT_, FULL_, MODE_) d2d_launch_step(d2d_step_warp_kernel<PLE2, EXACT_, WPB, FULL_, SPEC, MODE_>, grid, WPB * 32, smem, st, P, pdl)
+cudaError_t launch(const D2DParams &P, int grid, const D2DLaunchSel &sel, cudaStream_t st, bool pdl) {
+#define D2D_GO(EXACT_, FULL_, MODE_) d2d_launch_step(d2d_step_warp_kernel<PLE2, EXACT_, WPB, FULL_, SPEC, MODE_>, grid, WPB * 32, shape_smem(P.R), st, P, pdl)
     // (an episode's drawn positions are exact in fp32, so it never needs the fp64 shadow path)
     if (sel.episode && sel.fast && sel.full) return sel.no_reset ? D2D_GO(false, true, 4) : D2D_GO(false, true, 3);
     if (sel.episode) return D2D_GO(false, false, 2);
@@ -47,11 +49,8 @@ cudaError_t launch(const D2DParams &P, int grid, size_t smem, const D2DLaunchSel
     return sel.exact ? D2D_GO(true, false, 0) : D2D_GO(false, false, 0);
 #undef D2D_GO
 }
-}  // namespace
 
-size_t D2D_CAT(d2d_warp_smem_, D2D_TU_WPB)(int R) { return d2d_warp_smem_bytes(R, WPB); }
-
-int D2D_CAT(d2d_warp_plan_, D2D_TU_WPB)(d2d_handle *h, size_t smem) {
+int shape_plan(d2d_handle *h, size_t smem) {
     int rc;
     if (h->spec) {          // the reference's default EnvConfig shape: counts and division magics are immediates
         rc = allow_all<true, true>(smem);
@@ -66,22 +65,26 @@ int D2D_CAT(d2d_warp_plan_, D2D_TU_WPB)(d2d_handle *h, size_t smem) {
     return rc;
 }
 
-cudaError_t D2D_CAT(d2d_warp_launch_, D2D_TU_WPB)(const d2d_handle *h, const D2DParams &P, int grid, const D2DLaunchSel &sel, cudaStream_t st,
-                                                  bool pdl) {
-    if (h->spec) return launch<true, true>(P, grid, (size_t)sel.smem, sel, st, pdl);
-    if (h->ple2) return launch<true, false>(P, grid, (size_t)sel.smem, sel, st, pdl);
-    return launch<false, false>(P, grid, (size_t)sel.smem, sel, st, pdl);
+cudaError_t shape_launch(const d2d_handle *h, const D2DParams &P, int grid, const D2DLaunchSel &sel, cudaStream_t st, bool pdl) {
+    if (h->spec) return launch<true, true>(P, grid, sel, st, pdl);
+    if (h->ple2) return launch<true, false>(P, grid, sel, st, pdl);
+    return launch<false, false>(P, grid, sel, st, pdl);
 }
 
 // the fp64 pass reads 10^(p/10) from this translation unit's constant bank (per device: set at every d2d_create)
-cudaError_t D2D_CAT(d2d_warp_tables_, D2D_TU_WPB)(const double *pwr_lin_d) {
+cudaError_t shape_tables(const double *pwr_lin_d) {
     return cudaMemcpyToSymbol(d2d_pwr_lin_c, pwr_lin_d, sizeof(double) * D2D_MAX_PWR_LEVELS);
 }
 
 #ifdef D2D_TIMELINE
 // instrumented build (profiles/timeline.py): the stamp table is a __device__ variable of d2d_common.cuh, so every translation unit
 // has its own copy - the one this shape's kernels write is read here
-cudaError_t D2D_CAT(d2d_warp_timeline_, D2D_TU_WPB)(void *host_out, size_t bytes) {
+cudaError_t shape_timeline(void *host_out, size_t bytes) {
     return cudaMemcpyFromSymbol(host_out, d2d_tl_buf, bytes < sizeof(d2d_tl_buf) ? bytes : sizeof(d2d_tl_buf));
 }
+#else
+constexpr cudaError_t (*shape_timeline)(void *, size_t) = nullptr;
 #endif
+}  // namespace
+
+extern const D2DWarpShape D2D_CAT(d2d_warp_shape_, D2D_TU_WPB) = {WPB, shape_smem, shape_plan, shape_launch, shape_tables, shape_timeline};

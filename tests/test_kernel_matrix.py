@@ -1,6 +1,6 @@
 """GPU tier (-m gpu): every step-kernel instantiation d2d_create can pick, held to the float64 oracle.
 
-d2d_create (gym_d2d_b200/csrc/d2d_abi.cu:221-279) sends a configuration to one of four kernel families - the warp kernel
+d2d_create (gym_d2d_b200/csrc/d2d_abi.cu:223-279) sends a configuration to one of four kernel families - the warp kernel
 (2-, 4- or 8-warp blocks), the dense kernel (seven (links per thread, threads per block) shapes plus the instantiation for
 100 RBs / 100 CUEs / 500 DUE pairs), the sorting block kernel (1-4 links per thread) and the general-topology kernel - each
 instantiated for ple == 2 or not, and the dense and warp kernels also for the core-output (FULL) and fp64-shadow (EXACT)
